@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- V2CE hot path on B200: 346x260 frame-pairs/s (and LDATI Mevents/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1]): center 346x260, 321 synthetic gray frames = 20 windows of
 16 frame pairs, batch 4, random-init V2ce3d, voxel + LDATI + event-frame path.  One *step* is one
@@ -30,6 +30,11 @@ runs its own windows (weak scaling, windows are independent).
   sharded_parity   (N > 1) sharded event stream + preview == single-process, bit for bit, checked before timing
   cpu_baseline     the CPU oracle (torch-CPU fp32 UNet + numpy LDATI/EF restatement, oracle/) timed on
               the host cores on a bounded sample (1 window = 16 frame pairs); N = 1 only
+
+--dump-outputs DIR writes what the `value` path handed back in its last timed step (rank 0) as DIR/<name>.npy,
+float32 / float64, under 40 MB: the per-(pair, bin) event counts, a fixed seeded sample of the event records, the
+preview frames of a fixed seeded sample of the pairs and the preview's upper bound (dump_outputs).  Inputs, weights and
+seeds are fixed, so two builds run with the same arguments can be compared file by file.
 
 --impl reference times that CPU oracle port alone (the reference itself is Python and is not
 present on the GPU box; oracle/ is pinned to it by tests/golden).
@@ -168,9 +173,8 @@ def run_reference_arm(args, rank, world):
     if rank != 0:
         return
     units, _ = make_inputs()
-    # bounded: one window (16 pairs) per step; cap the step count so the arm ends within minutes
-    steps = max(1, min(args.steps, 6))
-    warmup = max(1, min(args.warmup, 1))
+    # one window (16 pairs) per step: a step takes seconds on the host cores
+    steps, warmup = args.steps, args.warmup
     pairs_s, mev_s, dt, cores = time_cpu_port(units, steps, warmup)
     line = {
         'impl': 'reference', 'metric': METRIC, 'value': pairs_s, 'unit': 'frame-pairs/s', 'n_gpus': args.gpus,
@@ -324,6 +328,32 @@ def check_sharded_parity(device, rank, world):
     return out
 
 
+DUMP_EVENTS = 1 << 20                  # event records sampled by --dump-outputs
+DUMP_PAIRS = 8                         # frame pairs whose preview frames --dump-outputs keeps
+
+
+def dump_outputs(out_dir, t):
+    """The results of BatchRunner ticket t as out_dir/<name>.npy: the event counts per (pair, bin), DUMP_EVENTS event
+    records at seeded sorted positions of the packed stream (all of them when there are fewer), the preview frames of
+    DUMP_PAIRS seeded pairs and the preview's upper bound.  Under 40 MB whatever the event count."""
+    from v2ce_toolbox_b200.ldati import EVENT_DTYPE
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    n = t.seg_counts.shape[0]
+    pairs = np.sort(rng.choice(n, min(n, DUMP_PAIRS), replace=False))
+    rows = np.arange(t.total) if t.total <= DUMP_EVENTS else np.sort(rng.choice(t.total, DUMP_EVENTS, replace=False))
+    packed = t.events_dev[:t.total * EVENT_DTYPE.itemsize].view(t.total, EVENT_DTYPE.itemsize)
+    ev = packed.index_select(0, torch.from_numpy(rows).to(packed.device)).cpu().numpy().reshape(-1).view(EVENT_DTYPE)
+    frames = t.frames_dev[torch.from_numpy(pairs).to(t.frames_dev.device)].cpu().numpy()
+    out = {'events_per_pair_bin': t.seg_counts.astype(np.float64), 'events_index': rows.astype(np.float64),
+           'events_timestamp': ev['timestamp'].astype(np.float64), 'events_x': ev['x'].astype(np.float32),
+           'events_y': ev['y'].astype(np.float32), 'events_polarity': ev['polarity'].astype(np.float32),
+           'event_frames_pairs': pairs.astype(np.float64), 'event_frames': frames.astype(np.float32),
+           'event_frames_upper_bound': np.array([t.ub], np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
     device = torch.device('cuda', local_rank)
@@ -350,7 +380,7 @@ def run_ours(args, rank, world, local_rank):
         computes."""
         br = r.host_runner if host_io else r.dev_runner
         src = r.units_pinned if host_io else r.units_dev
-        stats = {'events': 0, 'fwd': [], 'gap': [], 'h2d': 0, 'd2h': 0, 'last_fwd_end': None}
+        stats = {'events': 0, 'fwd': [], 'gap': [], 'h2d': 0, 'd2h': 0, 'last_fwd_end': None, 'last': None}
         pending = []                               # gathers in flight (their buffers alternate: wait for the one before last)
 
         def collect(t, timed):
@@ -378,6 +408,7 @@ def run_ours(args, rank, world, local_rank):
                 prev = t
             if prev is not None:
                 collect(prev, timed)
+                stats['last'] = prev
             while pending:
                 pending.pop(0).synchronize()
 
@@ -402,6 +433,8 @@ def run_ours(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     ms_dev, st_dev, launches = timed_loop(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, st_dev['last'])
     ms_e2e, st_e2e, _ = timed_loop(True)
     # the network alone (no event-frame / LDATI kernels sharing the SMs): what the roofline fraction describes
     fwd_ms = []
@@ -794,7 +827,13 @@ def main():
     ap.add_argument('--headline-only', action='store_true', help='skip the secondary records (ef, ldati, library, clips)')
     ap.add_argument('--long-frames', type=int, default=9000)
     ap.add_argument('--pano-frames', type=int, default=600)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the results of the last timed step as DIR/<name>.npy (see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the results of the CUDA path (--impl ours)')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))

@@ -3,15 +3,16 @@ batching, merge -- /root/reference/v2ce.py:45-239) against the UNMODIFIED refere
 
 Both drivers are handed the same stand-in for the network (a cheap deterministic map (b,L,2,H,W) -> (b,L,20,H,W) that
 also depends on the call index, like the real model's spectral-norm state) and the same in-memory clip, with
-``Tensor.cuda`` shimmed to the identity; every float of the merged voxel grid must agree.  Runs only where
-/root/reference is mounted."""
+``Tensor.cuda`` shimmed to the identity; every float of the merged voxel grid must agree.  The tests that import
+the reference run only where its sources are found (oracle/ref_harness.py, V2CE_REFERENCE_ROOT)."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import ref_harness as rh, synth
 
-pytestmark = pytest.mark.skipif(not rh.available(), reason='/root/reference is not mounted')
+needs_reference = pytest.mark.skipif(not rh.available(), reason='the upstream V2CE-Toolbox sources are not found '
+                                                                 '(set V2CE_REFERENCE_ROOT)')
 
 
 class StandIn(torch.nn.Module):
@@ -40,6 +41,7 @@ CASES = [('center', 16, 1, 26, 40, 36),                       # one window start
          ('pano', 33, 1, 52, 104, 20)]                        # resized, 3 tiles, the last one pulled back
 
 
+@needs_reference
 @pytest.mark.parametrize('infer_type,n_frames,batch_size,H,W,width', CASES)
 def test_video_to_voxels_equals_reference_driver(infer_type, n_frames, batch_size, H, W, width):
     from v2ce_toolbox_b200 import v2ce as drv
@@ -83,6 +85,7 @@ def _write_mp4(path, n_frames, H, W, seed=0):
     return frames
 
 
+@needs_reference
 def test_video_reader_equals_reference_reader(tmp_path):
     """scripts/video_reader.py as the CLI uses it (v2ce.py:333-335,170): same frame count and the same gray frames for
     the index patterns the driver issues -- consecutive windows, the one-frame overlap between windows, a pulled-back
@@ -111,6 +114,7 @@ def test_video_reader_equals_reference_reader(tmp_path):
     ours.close()
 
 
+@needs_reference
 def test_cli_flags_equal_the_reference_parser():
     """Drop-in boundary (SURVEY.md 8b): every flag of the reference's argparse block (v2ce.py:283-302), with its option
     strings, type, default, nargs and const, exists unchanged in the product's parser; the product adds only --seed."""
@@ -141,6 +145,7 @@ def test_cli_flags_equal_the_reference_parser():
     assert set(ours) - set(ref) == {('--seed',)}
 
 
+@needs_reference
 def test_drop_in_signatures_equal_the_reference():
     """Same names, positional order and defaults for every callable of the boundary (SURVEY.md 8b); the product may add
     keyword-only extensions (seed / frame_base / draws / flavor on sample_voxel_statistical) and nothing else."""

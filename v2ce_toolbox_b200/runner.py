@@ -52,7 +52,7 @@ def nvtx(name):
 class Ticket:
     __slots__ = ('slot', 'n_pairs', 'total', 'seg_counts', 'done', 'status', 'ub', 'h2d_bytes', 'd2h_bytes', 'hw',
                  'pair_base', 'vox', 'sums', 'small_host', 'counts_ready', 'staged', 'params', 'offs', 'fwd_events',
-                 'events_dev', 'packed', 'ev_host')
+                 'events_dev', 'frames_dev', 'packed', 'ev_host')
 
 
 class BatchRunner:
@@ -257,6 +257,7 @@ class BatchRunner:
             _, status = eng.emit(t.vox, t.params, total, frame_offsets=t.offs, out=ev, status_out=st_dev)
             self.launches += eng.launches - l0
             t.events_dev = ev
+            t.frames_dev = frames
             t.packed = torch.cuda.Event()
             t.packed.record(self.post_stream)
         t.d2h_bytes = 0
@@ -334,7 +335,7 @@ class BatchRunner:
 
     def wait(self, t, copy=True):
         """Block until batch `t` is on the host.  Returns (events recarray view, frames uint8 (n,H,W,3) | None);
-        with copy_out=False both are None (results stay in the slot's device buffers)."""
+        with copy_out=False both are None (results stay in the slot's device buffers, t.events_dev / t.frames_dev)."""
         self._stage_b(t)
         t.done.synchronize()
         _ldati.check_status(t.status.numpy())
