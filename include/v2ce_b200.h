@@ -209,6 +209,10 @@ int v2ce_model_set_tensor(v2ce_model* m, const char* name, const float* data_hos
 int v2ce_model_finalize(v2ce_model* m);
 int v2ce_model_workspace_bytes(const v2ce_model* m, int32_t batch, int32_t depth, int32_t height,
                                int32_t width, size_t* bytes);
+/* Byte offsets into the workspace of its bf16 activation buffers at this shape (per-layer tests), in this order:
+ * head_in, head, enc0..3, res0..1, dec0..3, tmp_t, tmp_r, up, up2 (16 entries; cap must be >= 16, *n receives 16). */
+int v2ce_model_workspace_layout(const v2ce_model* m, int32_t batch, int32_t depth, int32_t height, int32_t width,
+                                int64_t* offsets, int32_t cap, int32_t* n);
 /* x_dev (B,L,2,H,W) float32 -> y_dev (B,L,20,H,W) float32 (v2ce_3d.py:26-30).  Advances the
  * spectral-norm power iteration by one step, as the reference does on every forward. */
 int v2ce_model_forward(v2ce_model* m, const float* x_dev, float* y_dev, int32_t batch, int32_t depth,
@@ -223,7 +227,7 @@ int v2ce_model_forward_frames(v2ce_model* m, const uint8_t* frames_dev, float* y
 int v2ce_model_last_sigmas(const v2ce_model* m, float* sigma12_host);
 int v2ce_model_call_count(const v2ce_model* m, int64_t* calls);
 int v2ce_model_sn_advance(v2ce_model* m, int32_t n_calls, void* stream);
-/* Number of kernels the last forward launched (bench.py's gpu_launches). */
+/* Number of kernels the last complete forward launched (bench.py's gpu_launches). */
 int v2ce_model_last_launches(const v2ce_model* m, int32_t* launches);
 
 /* Layer-level hook used by the parity tests: one fused conv launch.
@@ -251,7 +255,10 @@ int v2ce_debug_mma_rate(int32_t bn, int32_t iters, int32_t naccs, int32_t ctas, 
 /* Per-launch device times of the last forward, measured with CUDA events on the launch stream when the option
  * "layer_timing" is 1: ms_out[i] and the layer name (48 bytes each, NUL terminated) of launch i. */
 int v2ce_model_layer_times(v2ce_model* m, int32_t cap, float* ms_out, char* names_out, int32_t* count);
-/* Tuning / bring-up options of a model handle: "desc_mode", "layer_timing". */
+/* Tuning / bring-up options of a model handle: "desc_mode", "layer_timing", and "stop_after" (per-layer tests; default
+ * -1 = off): a layer index in state-dict order (head 0 .. pred 31); the forward returns right after the launch that
+ * writes that layer's output, with every stream it used joined into `stream`.  A block's shortcut fused into its conv1
+ * stops after that launch, pred after decoders.3.conv2.  The workspace then holds the layer's inputs and its output. */
 int v2ce_model_set_option(v2ce_model* m, const char* key, int64_t value);
 
 /* ------------------------------------------------------------------------------------------

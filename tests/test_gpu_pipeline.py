@@ -36,11 +36,15 @@ def test_video_to_voxels_matches_reference_golden(name, golden, golden_meta):
     assert rel <= 1.6e-2, rel                                 # 'lively' stress weights: see tests/test_gpu_unet.py
 
 
-@pytest.mark.parametrize('n_frames,bs', [(20, 2), (33, 1), (36, 4)])
-def test_stream_clip_events_and_frames_bit_exact_on_device_voxels(n_frames, bs):
+@pytest.mark.parametrize('n_frames,bs,seq_len', [pytest.param(20, 2, 16, id='20-2'), pytest.param(33, 1, 16, id='33-1'),
+                                                 pytest.param(36, 4, 16, id='36-4'),
+                                                 # --seq_len 10 / 8 with the last window pulled back
+                                                 pytest.param(26, 2, 10, id='26-2-seq10'),
+                                                 pytest.param(21, 3, 8, id='21-3-seq8')])
+def test_stream_clip_events_and_frames_bit_exact_on_device_voxels(n_frames, bs, seq_len):
     """The CLI path (voxels never leave the GPU) must produce exactly what the reference's steps produce
     from the same voxels: event frames and the offset, concatenated event stream."""
-    _check_stream_clip(n_frames, bs)
+    _check_stream_clip(n_frames, bs, seq_len=seq_len)
 
 
 @pytest.mark.parametrize('n_frames,bs', [(16, 1), (2, 1), (3, 2), (17, 4)])
@@ -66,12 +70,12 @@ def test_stream_clip_image_folders_incl_tiny_ones(n_frames, bs, tmp_path):
     _check_stream_clip(n_frames, bs, image_paths=paths)
 
 
-def _check_stream_clip(n_frames, bs, image_paths=None):
+def _check_stream_clip(n_frames, bs, image_paths=None, seq_len=16):
     from v2ce_toolbox_b200 import v2ce as drv
     H, W = 28, 36
     frames = synth.make_video(n_frames, H, W, seed=9)
     src = dict(image_paths=image_paths) if image_paths is not None else dict(vidcap=FakeVideoReader(frames))
-    vox = drv.video_to_voxels(_model(6), infer_type='center', seq_len=16, width=W, height=H, batch_size=bs, **src)
+    vox = drv.video_to_voxels(_model(6), infer_type='center', seq_len=seq_len, width=W, height=H, batch_size=bs, **src)
     vox = vox * np.float32(3)                                 # the check below feeds the same scaled voxels to both sides
     if image_paths is None:
         assert vox.shape[0] == n_frames - 1
@@ -85,7 +89,7 @@ def _check_stream_clip(n_frames, bs, image_paths=None):
             return self.inner(x) * 3.0
 
     src = dict(image_paths=image_paths) if image_paths is not None else dict(vidcap=FakeVideoReader(frames))
-    res = drv.stream_clip(Scaled(_model(6)), infer_type='center', seq_len=16, width=W,
+    res = drv.stream_clip(Scaled(_model(6)), infer_type='center', seq_len=seq_len, width=W,
                           height=H, batch_size=bs, fps=30, ceil=10, upper_bound_percentile=98, seed=77, **src)
     assert res.n_pairs == vox.shape[0]
     want_frames, want_ub, _ = ef_oracle.event_frames_oracle(vox, 10, 98, True)

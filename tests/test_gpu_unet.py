@@ -167,7 +167,11 @@ def _model(seed, init):
 
 
 @pytest.mark.parametrize('init,shape', [('lively', (1, 16, 2, 36, 44)), ('lively', (2, 16, 2, 20, 28)),
-                                        ('reference', (1, 16, 2, 65, 87)), ('lively', (1, 16, 2, 260, 346))])
+                                        ('reference', (1, 16, 2, 65, 87)), ('lively', (1, 16, 2, 260, 346))] +
+                         # the other schedules: depth-merged at T=8 only, the seq_len % 8 != 0 schedule (direct head,
+                         # gather, conv_halo T=2), three depth groups, the one-pixel bottleneck
+                         [(init, shape) for shape in ((1, 8, 2, 40, 52), (2, 10, 2, 36, 44), (1, 24, 2, 36, 44),
+                                                      (2, 16, 2, 8, 12)) for init in ('lively', 'reference')])
 def test_forward_vs_fp32_oracle(init, shape):
     """Tolerance (stated, SURVEY.md F10): bf16 operands / fp32 accumulation / bf16 inter-layer activations against the
     fp32 reference, on two consecutive calls (spectral-norm state).  With the reference's own initialisation (what every
@@ -237,23 +241,25 @@ def test_forward_frames_equals_forward_of_preprocessed_units():
     H, W = 36, 44
     frames = synth.make_video(35, H, W, seed=4)
     frames[0, 0, :4] = (0, 1, 254, 255)                      # the ends of the gray range
-    wins = np.stack([frames[0:17], frames[16:33]], axis=0)   # two windows
-    units = torch.stack([image_pre_processing(w, H) for w in wins], dim=0)
-    m1, _ = _model(2, 'lively')
-    m2, _ = _model(2, 'lively')
-    y_units = m1(units.cuda())
-    y_frames = m2.forward_frames(torch.from_numpy(wins).cuda())
-    assert torch.equal(y_units, y_frames)
+    # two 16-pair windows (tensor-pipe head) and one of 10 pairs (direct head, head_conv_kernel<true> against <false>)
+    for wins in (np.stack([frames[0:17], frames[16:33]], axis=0), frames[None, 0:11]):
+        units = torch.stack([image_pre_processing(w, H) for w in wins], dim=0)
+        m1, _ = _model(2, 'lively')
+        m2, _ = _model(2, 'lively')
+        y_units = m1(units.cuda())
+        y_frames = m2.forward_frames(torch.from_numpy(np.ascontiguousarray(wins)).cuda())
+        assert torch.equal(y_units, y_frames), wins.shape
 
 
 def test_full_size_batch_is_per_window_deterministic():
     """BASELINE configs[1] shape (batch 4, 346x260): every window of a batch equals the same window run alone, bit for
     bit (tiles never mix batch items; no atomics in the conv path), on two consecutive calls of the SN schedule."""
-    m4, _ = _model(9, 'lively')
-    m1, _ = _model(9, 'lively')
-    g = torch.Generator(device='cpu').manual_seed(1)
-    x = torch.randn(4, 16, 2, 260, 346, generator=g).cuda()
-    y4 = m4(x)
-    y1 = m1(x[2:3].contiguous())
-    assert torch.isfinite(y4).all() and (y4 >= 0).all()
-    assert torch.equal(y4[2:3], y1)
+    for B, D, k in ((4, 16, 2), (3, 10, 1)):                 # (3, 10): the seq_len % 8 != 0 schedule
+        mb, _ = _model(9, 'lively')
+        m1, _ = _model(9, 'lively')
+        g = torch.Generator(device='cpu').manual_seed(1)
+        x = torch.randn(B, D, 2, 260, 346, generator=g).cuda()
+        yb = mb(x)
+        y1 = m1(x[k:k + 1].contiguous())
+        assert torch.isfinite(yb).all() and (yb >= 0).all()
+        assert torch.equal(yb[k:k + 1], y1), (B, D)

@@ -78,6 +78,8 @@ _SIGNATURES = {
     'v2ce_model_set_tensor': (c_int, [c_void_p, c_char_p, c_void_p, POINTER(c_int64), c_int32]),
     'v2ce_model_finalize': (c_int, [c_void_p]),
     'v2ce_model_workspace_bytes': (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, POINTER(c_size_t)]),
+    'v2ce_model_workspace_layout': (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, POINTER(c_int64), c_int32,
+                                            POINTER(c_int32)]),
     'v2ce_model_forward': (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p,
                                    c_size_t, c_void_p]),
     'v2ce_model_forward_frames': (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p,

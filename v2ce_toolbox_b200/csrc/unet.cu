@@ -450,6 +450,7 @@ struct v2ce_model {
   int last_launches = 0;
   int desc_mode = 0;
   int layer_timing = 0;                 // option "layer_timing": CUDA events around every launch of forward()
+  int stop_after = -1;                  // option "stop_after" (per-layer tests): kLayers index, -1 = run the whole forward
   std::vector<std::pair<std::string, cudaEvent_t>> marks;
   cudaStream_t sn_stream = nullptr;     // the spectral-norm step overlaps the head / encoder convs
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
@@ -949,6 +950,21 @@ extern "C" int v2ce_model_workspace_bytes(const v2ce_model* m, int32_t batch, in
   return V2CE_OK;
 }
 
+extern "C" int v2ce_model_workspace_layout(const v2ce_model* m, int32_t batch, int32_t depth, int32_t height, int32_t width,
+                                           int64_t* offsets, int32_t cap, int32_t* n) {
+  V2CE_REQUIRE(m && offsets && n, "NULL argument");
+  V2CE_REQUIRE(batch > 0 && depth > 0 && height > 0 && width > 0, "bad shape");
+  V2CE_REQUIRE((long long)batch * depth * height * width < (1LL << 31), "batch*depth*H*W must be < 2^31");
+  const Buffers b = carve(nullptr, make_dims(batch, depth, height, width));
+  const __nv_bfloat16* p[] = {b.head_in, b.head, b.enc[0], b.enc[1], b.enc[2], b.enc[3], b.res[0], b.res[1],
+                              b.dec[0], b.dec[1], b.dec[2], b.dec[3], b.tmp_t, b.tmp_r, b.up, b.up2};
+  constexpr int kBufs = sizeof(p) / sizeof(p[0]);
+  V2CE_REQUIRE(cap >= kBufs, "offsets holds %d entries, the layout has %d", cap, kBufs);
+  for (int i = 0; i < kBufs; ++i) offsets[i] = (int64_t)reinterpret_cast<uintptr_t>(p[i]);
+  *n = kBufs;
+  return V2CE_OK;
+}
+
 static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float* y_dev, int32_t B, int32_t D, int32_t H,
                         int32_t W, void* ws_dev, size_t ws_bytes, void* stream) {
   V2CE_REQUIRE(m && x_dev && y_dev && ws_dev, "NULL argument");
@@ -971,6 +987,15 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     m->marks[n_marks].first = what;
     cudaEventRecord(m->marks[n_marks].second, s);
     ++n_marks;
+  };
+  // option "stop_after": return right after the launch that writes layer stop_after's output (a block's shortcut fused
+  // into its conv1 stops there, pred stops after decoders.3.conv2), with the side stream joined into `s`.  Every launch
+  // writes out of place, so the workspace then holds both the inputs of that layer and its output.
+  auto stop_at = [&](int l0, int l1) { return m->stop_after >= 0 && (m->stop_after == l0 || m->stop_after == l1); };
+  auto stop = [&]() -> int {
+    V2CE_CUDA_CHECK(cudaEventRecord(m->ev_join, m->sn_stream));
+    V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_join, 0));
+    return V2CE_OK;
   };
   mark("start");
   // spectral-norm power iteration (input independent) on a side stream, joined before the first SN conv
@@ -1040,6 +1065,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
   }
   ++launches;
   mark("UNet.head.conv3d");
+  if (stop_at(0, -1)) return stop();
 
   static const int ch[5] = {32, 64, 128, 256, 512};
   char name[64];
@@ -1054,14 +1080,18 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     if (fused) {
       mark(kLayers[l1].name);
       launches -= 1;
+      if (stop_at(l1, l1 + 2)) return stop();
     } else {
       if (int e = run_conv(m, l1, x, pin, d.H[i], d.W[i], nullptr, 0, B, D, d.H[i], d.W[i], 2, nullptr, 1, buf.tmp_t, s)) return e;
       mark(kLayers[l1].name);
+      if (stop_at(l1, -1)) return stop();
       if (int e = run_conv(m, l1 + 2, x, pin, d.H[i], d.W[i], nullptr, 0, B, D, d.H[i], d.W[i], 2, nullptr, 0, buf.tmp_r, s)) return e;
       mark(kLayers[l1 + 2].name);
+      if (stop_at(l1 + 2, -1)) return stop();
     }
     if (int e = run_halo(m, l1 + 1, buf.tmp_t, co, nullptr, 0, B, D, d.H[i + 1], d.W[i + 1], buf.tmp_r, co, 1, buf.enc[i], co, s)) return e;
     mark(kLayers[l1 + 1].name);
+    if (stop_at(l1 + 1, -1)) return stop();
     x = buf.enc[i];
     launches += 3;
   }
@@ -1082,6 +1112,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     }
     if (int e = run_halo(m, l1, x, 512, nullptr, 0, B, D, d.H[4], d.W[4], nullptr, 0, 1, buf.tmp_t, 512, s)) return e;
     mark(kLayers[l1].name);
+    if (stop_at(l1, -1)) return stop();
     if (int e = run_conv(m, l1 + 2, x, 512, d.H[4], d.W[4], nullptr, 0, B, D, d.H[4], d.W[4], 1, nullptr, 0, buf.tmp_r,
                          side ? m->sn_stream : s)) return e;
     mark(kLayers[l1 + 2].name);
@@ -1090,6 +1121,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
       V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_side[side_ev + 1], 0));
       side_ev += 2;
     }
+    if (stop_at(l1 + 2, -1)) return stop();
     // the last block's output is only ever read nearest-upsampled by decoders.0: write it that way
     if (i == 1) {
       if (int e = run_halo(m, l1 + 1, buf.tmp_t, 512, nullptr, 0, B, D, d.H[4], d.W[4], buf.tmp_r, 512, 1, buf.up, 512, s,
@@ -1098,6 +1130,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
       if (int e = run_halo(m, l1 + 1, buf.tmp_t, 512, nullptr, 0, B, D, d.H[4], d.W[4], buf.tmp_r, 512, 1, buf.res[i], 512, s)) return e;
     }
     mark(kLayers[l1 + 1].name);
+    if (stop_at(l1 + 1, -1)) return stop();
     x = buf.res[i];
     launches += 3;
   }
@@ -1122,6 +1155,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     if (int e = run_halo(m, l1, up_cur, xc, skip, sp, B, D, d.H[lvl], d.W[lvl], nullptr, 0, 1, buf.tmp_t, tp, s, 0, 0, nullptr,
                          l1 + 2, buf.tmp_r, co, &short_done)) return e;
     mark(kLayers[l1].name);
+    if (stop_at(l1, short_done ? l1 + 2 : -1)) return stop();
     if (!short_done) {
       if (int e = run_conv(m, l1 + 2, up_cur, xc, d.H[lvl], d.W[lvl], skip, sp, B, D, d.H[lvl], d.W[lvl], 1, nullptr, 0, buf.tmp_r,
                            side ? m->sn_stream : s)) return e;
@@ -1131,6 +1165,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
         V2CE_CUDA_CHECK(cudaEventRecord(m->ev_side[side_ev + 1], m->sn_stream));
         V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_side[side_ev + 1], 0));
       }
+      if (stop_at(l1 + 2, -1)) return stop();
     }
     if (side) side_ev += 2;
     if (lvl > 0) {
@@ -1141,6 +1176,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
                            0, 0, y_dev)) return e;
     }
     mark(kLayers[l1 + 1].name);
+    if (stop_at(l1 + 1, lvl == 0 ? kNumLayers - 1 : -1)) return stop();
     __nv_bfloat16* tsw = up_cur; up_cur = up_next; up_next = tsw;
     xc = co;
     launches += 2;
@@ -1208,6 +1244,11 @@ extern "C" int v2ce_model_set_option(v2ce_model* m, const char* key, int64_t val
   V2CE_REQUIRE(m && key, "NULL argument");
   if (std::string(key) == "desc_mode") { m->desc_mode = (int)value; return V2CE_OK; }
   if (std::string(key) == "layer_timing") { m->layer_timing = (int)value; return V2CE_OK; }
+  if (std::string(key) == "stop_after") {
+    V2CE_REQUIRE(value >= -1 && value < kNumLayers, "stop_after must be -1 or a layer index < %d", kNumLayers);
+    m->stop_after = (int)value;
+    return V2CE_OK;
+  }
   return set_error(V2CE_ERR_INVALID, "unknown option '%s'", key);
 }
 
