@@ -117,26 +117,6 @@ def test_full_size_digest_matches_reference_sparse(golden_meta):
     assert hashlib.sha256(c.tobytes()).hexdigest() == m['sha256'][0]
 
 
-def test_size_independent_properties_full_config():
-    """BASELINE config 3 shape (dense counts, 24-frame chunk): conservation, ranges, sortedness."""
-    F, H, W = 24, 260, 346
-    v = synth.make_voxels('randint', F, H, W, seed=8)
-    got = _run(v, fps=30, seed=1)
-    n, _ = lo.relocate_counts(v)
-    per_frame = np.clip(n, 0, None).reshape(F, -1).sum(axis=1)
-    assert [len(g) for g in got] == per_frame.tolist()
-    seg = np.clip(n, 0, None).sum(axis=(1, 3, 4))            # (F,9)
-    for f in (0, 11, 23):
-        e = got[f]
-        assert e['x'].min() >= 0 and e['x'].max() < W and e['y'].min() >= 0 and e['y'].max() < H
-        start = 0
-        for c in range(9):
-            ts = e['timestamp'][start:start + seg[f, c]]
-            assert (np.diff(ts) >= 0).all()
-            assert ts.min() >= int(c * 1e6 / 30 / 9) - 2 and ts.max() <= int((c + 1) * 1e6 / 30 / 9) + 2
-            start += seg[f, c]
-
-
 def test_rejects_cpu_tensor_and_unsupported_modes():
     from v2ce_toolbox_b200 import V2ceError
     from v2ce_toolbox_b200.scripts.LDATI import sample_voxel_statistical

@@ -59,7 +59,7 @@ def test_kernels_equal_torch_cuda_options(kind, opts):
     _compare(_vox(kind, 2, 37, 53, 7), **opts)
 
 
-@pytest.mark.parametrize('fps', [24, 60, 120, 1000])
+@pytest.mark.parametrize('fps', [1, 5, 10, 24, 60, 120, 1000])
 def test_kernels_equal_torch_cuda_frame_rates(fps):
     _compare(_vox('mixed', 1, 64, 96, fps), fps=fps)
 

@@ -11,7 +11,7 @@ pytestmark = pytest.mark.gpu
 F32 = np.float32
 
 
-@pytest.mark.parametrize('fps', [24, 25, 30, 50, 60, 120, 240, 1000])
+@pytest.mark.parametrize('fps', [1, 5, 10, 24, 25, 30, 50, 60, 120, 240, 1000])
 def test_arange_bin_starts(fps):
     got = torch.arange(0, 1 / fps, 1 / fps / 9, device='cuda').cpu().numpy()
     assert got.dtype == np.float32
@@ -22,7 +22,7 @@ def test_division_by_python_scalar_is_reciprocal_multiply():
     g = torch.Generator(device='cpu').manual_seed(0)
     x32 = torch.rand(1 << 16, generator=g)
     x64 = x32.double()
-    for fps in (24, 30, 120):
+    for fps in (1, 5, 10, 24, 30, 120):
         k = lo.Consts(fps, 0, 'cuda')
         got = (x64.cuda() / fps / 9).cpu().numpy()
         assert np.array_equal(got, x64.numpy() * k.r_fps64 * k.r_c64)
