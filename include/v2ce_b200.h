@@ -46,8 +46,8 @@ int v2ce_device_check(int device, int* sm_count, int* cc_major, int* cc_minor);
  * pick_elements (:217-245) and pick_and_sort (:248-310).  The configuration v2ce.py:356 uses
  * (bidirectional=False, additional_events_strategy='slope', pooling_type='none') is the tuned path;
  * bidirectional=True and the 'random' / 'none' strategies are implemented as options of the same
- * kernels, and so is pooling_type 'avg' / 'weighted' (the Python shim still raises for it unless
- * V2CE_EXPERIMENTAL_POOLING=1: that route has not run on hardware yet).
+ * kernels, and so is pooling_type 'avg' / 'weighted' (the slope is fitted on pooled counts; the Python
+ * shim accepts every pooling_type the reference does).
  *
  * The scalar constants are computed by the host with the reference's own Python
  * expressions (SURVEY.md Appendix A) so the kernel reproduces torch's rounding.

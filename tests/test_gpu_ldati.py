@@ -165,42 +165,19 @@ def test_options_cpu_flavour_against_reference_goldens(name, golden, golden_meta
             assert d.max() <= 1 and (d != 0).mean() <= 1e-3
 
 
-@pytest.fixture
-def ldati_variant(monkeypatch):
-    """Sets the per-call opt-in switches of csrc/ldati.cu (read with getenv on every emit call)."""
-    def set_(reuse, staged, onesweep=1):
-        monkeypatch.setenv('V2CE_LDATI_REUSE_WARP_TOTALS', str(int(reuse)))
-        monkeypatch.setenv('V2CE_LDATI_STAGED_SCATTER', str(int(staged)))
-        monkeypatch.setenv('V2CE_LDATI_ONESWEEP', str(int(onesweep)))
-    return set_
-
-
-VARIANT_CASES = [('randint', 2, 24, 30, {}), ('mixed', 2, 33, 47, {}), ('rand', 1, 260, 346, {}),
-                 ('randint', 1, 260, 346, {}), ('mixed', 2, 40, 52, dict(additional_events_strategy='random')),
-                 ('mixed', 2, 33, 47, dict(bidirectional=True)),
-                 ('sparse', 3, 40, 52, dict(additional_events_strategy='none'))]
-_variant_oracle = {}
-
-
-def _variant_case(i):
-    if i not in _variant_oracle:
-        kind, F, H, W, opts = VARIANT_CASES[i]
-        v = synth.make_voxels(kind, F, H, W, seed=51)
-        _variant_oracle[i] = (v, lo.sample_voxel_statistical_oracle(v, fps=30, seed=9, frame_base=2, flavor='cuda', **opts))
-    return _variant_oracle[i]
-
-
-@pytest.mark.parametrize('reuse,staged,onesweep', [(0, 0, 0), (1, 0, 0), (0, 1, 0), (1, 1, 0), (0, 0, 1), (1, 1, 1)])
-def test_kernel_variants_bit_exact(reuse, staged, onesweep, ldati_variant):
-    """The kernel variants, every on/off combination (per-warp totals handed from the count pass to the emit pass; sort tiles ordered
-    by digit in shared memory before the scatter) produce the same bytes as the oracle: dense, sparse and mixed
-    counts, V=1 and V=4 pixel paths, 32- and 64-bit elements, 2- and 3-pass sorts, both relocation directions."""
-    ldati_variant(reuse, staged, onesweep)
-    for i, (kind, F, H, W, opts) in enumerate(VARIANT_CASES):
-        v, want = _variant_case(i)
-        got = _run(v, fps=30, seed=9, frame_base=2, **opts)
-        for j, (g, w) in enumerate(zip(got, want)):
-            _assert_rows_equal(g, w, f'reuse={reuse} staged={staged} onesweep={onesweep} {kind} {opts} frame {j}')
+@pytest.mark.parametrize('kind,F,H,W,opts', [
+    ('randint', 2, 24, 30, {}), ('mixed', 2, 33, 47, {}), ('rand', 1, 260, 346, {}), ('randint', 1, 260, 346, {}),
+    ('mixed', 2, 40, 52, dict(additional_events_strategy='random')), ('mixed', 2, 33, 47, dict(bidirectional=True)),
+    ('sparse', 3, 40, 52, dict(additional_events_strategy='none'))])
+def test_emit_sort_and_pack_bit_exact(kind, F, H, W, opts):
+    """Emit pass (per-warp totals handed over by the count pass), one-sweep sort and record writer produce the same
+    bytes as the oracle: dense, sparse and mixed counts, V=1 and V=4 pixel paths, 32- and 64-bit elements, 2- and
+    3-pass sorts, both relocation directions."""
+    v = synth.make_voxels(kind, F, H, W, seed=51)
+    want = lo.sample_voxel_statistical_oracle(v, fps=30, seed=9, frame_base=2, flavor='cuda', **opts)
+    got = _run(v, fps=30, seed=9, frame_base=2, **opts)
+    for j, (g, w) in enumerate(zip(got, want)):
+        _assert_rows_equal(g, w, f'{kind} {opts} frame {j}')
 
 
 def test_bidirectional_tendency_beyond_sort_window_raises():

@@ -12,7 +12,6 @@ import json
 d=json.load(open('$OUT/ldati_table.json'))
 for k,v in d.items(): print(k, round(v['ms'],3), 'ms', round(v['frac_of_hbm_peak'],3))
 "
-V2CE_LDATI_ONESWEEP=0 timeout 120 python tools/ldati_bench.py 5 --pairs 24 --dist rand > "$OUT/ldati_rand_oldsort.json" 2>&1
 for d in rand randint10 sparse; do
   timeout 200 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file "$OUT/ldati_launches_$d.csv" \
       python tools/ldati_bench.py 1 --pairs 24 --dist $d > "$OUT/ldati_$d.log" 2>&1

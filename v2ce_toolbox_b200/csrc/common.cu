@@ -23,11 +23,6 @@ int device_slot() {
   return dev & 63;
 }
 
-bool pdl_enabled() {
-  static const bool on = getenv("V2CE_PDL") && atoi(getenv("V2CE_PDL")) != 0;   // measured: no gain (9.4 ms either way), off by default
-  return on;
-}
-
 int sm_count_cached() {
   static int cached = 0;
   if (cached == 0) {

@@ -52,34 +52,8 @@ struct Arena {
 };
 
 int sm_count_cached();
-// Programmatic dependent launch: a conv kernel is launched while its predecessor on the stream is still draining;
-// its CTAs become resident as the predecessor's CTAs exit and run their prologue (mbarrier init, TMEM allocation,
-// tensor-map fetch) before `griddepcontrol.wait` holds them until the predecessor's memory is visible.
-// Opt-in with V2CE_PDL=1 (measured on B200: no gain for this network, the launch gaps are not what the forward waits
-// for); without the launch attribute the device instructions are no-ops.
-bool pdl_enabled();
 // index (< 64) of the current CUDA device: function attributes and constant memory are per device, so the
 // one-time-setup caches of the launchers are kept per device (one process may drive several GPUs)
 int device_slot();
-
-#ifdef __CUDACC__
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t s, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3((unsigned)block);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-#endif
 
 }  // namespace v2ce

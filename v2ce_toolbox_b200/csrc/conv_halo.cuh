@@ -28,7 +28,6 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 #include "conv_igemm.cuh"
 
@@ -280,9 +279,6 @@ __global__ void __launch_bounds__(kHaloThreads) conv_halo_kernel(const __grid_co
   __syncthreads();
   tcgen05_fence_after();
   const uint32_t tmem_acc = *tmem_ptr;
-  // prologue done: let the next kernel of the stream be launched, then wait for the previous one's results
-  pdl_launch_dependents();
-  pdl_wait();
 
   // Persistent CTA: every role walks the same tile sequence; the smem rings and their phases run on
   // across tiles, so the producers prefetch the next tile while the current one is multiplied/stored.
@@ -340,7 +336,7 @@ __global__ void __launch_bounds__(kHaloThreads) conv_halo_kernel(const __grid_co
       tcgen05_fence_after();
       const uint32_t acc_base = tmem_acc + (uint32_t)(ab * T * BN);
       for (int cc = 0; cc < ncc; ++cc) {
-        // zero-padded channels (64-channel pitch of a 32-channel tensor) are not multiplied
+        // channels beyond the real ones (the upper half of a 32-channel tensor's 64-channel rows) are not multiplied
         const int rem = (cc < a.ncc0) ? (a.real0 - cc * kBlockK) : (a.real1 - (cc - a.ncc0) * kBlockK);
         const int ks = rem >= kBlockK ? kBlockK / 16 : (rem + 15) / 16;
 #pragma unroll 1
@@ -532,9 +528,6 @@ struct TileShape { int PW, TH; };
 // pitch / rows per tile for an output plane of H x W (see file header); chosen to maximise the useful
 // fraction of the 128 accumulator rows
 inline TileShape pick_tile(int H, int W) {
-  // tuning override for the large planes: V2CE_TILE_PW=<patch pitch>
-  static const int force_pw = getenv("V2CE_TILE_PW") ? atoi(getenv("V2CE_TILE_PW")) : 0;
-  if (force_pw >= 4 && W >= 100) return TileShape{force_pw, 128 / force_pw};
   TileShape best{16, 8};
   double best_eff = 0.0;
   for (int pw = 10; pw <= 66; pw += 2) {
@@ -564,23 +557,16 @@ inline HaloPlan plan_for(int bn, int D, int H, int W) {
   const int b_stage = bn * kBlockK * 2;
   // depth blocking T and ring depths.  A chunk needs T patches before its first tap and holds T+2 over its
   // lifetime; the ring must be deep enough to prefetch the next chunk's first patches (SA >= T + 2 + T/2 would
-  // be ideal), which T = 2 allows within 227 KB while T = 4 does not.  Tuning knobs: V2CE_HALO_T / _SA / _SB.
-  const char* et = getenv("V2CE_HALO_T");
-  const char* esa = getenv("V2CE_HALO_SA");
-  const char* esb = getenv("V2CE_HALO_SB");
-  p.T = et ? atoi(et) : (bn <= 64 ? 4 : 2);   // measured: T=4 wins for N<=64, T=2 (double-buffered TMEM) for N=128
-  if (bn > 128 && p.T > 2) p.T = 2;
+  // be ideal), which T = 2 allows within 227 KB while T = 4 does not.
+  p.T = bn <= 64 ? 4 : 2;   // measured: T=4 wins for N<=64, T=2 (double-buffered TMEM) for N=128
   while (p.T > 1 && (D % p.T != 0)) p.T /= 2;
   for (;; p.T /= 2) {
-    p.SB = esb ? atoi(esb) : (bn <= 32 ? 8 : bn <= 64 ? 6 : bn <= 128 ? 4 : 3);
-    p.SA = esa ? atoi(esa) : kMaxSA;
-    if (p.SA > kMaxSA) p.SA = kMaxSA;
-    if (p.SB > kMaxSB) p.SB = kMaxSB;
+    p.SB = bn <= 32 ? 8 : bn <= 64 ? 6 : bn <= 128 ? 4 : 3;
+    p.SA = kMaxSA;
     while (p.SA > p.T + 1 && p.SA * p.a_stage_bytes + p.SB * b_stage > budget) --p.SA;
     while (p.SB > 2 && p.SA * p.a_stage_bytes + p.SB * b_stage > budget) --p.SB;
     if (p.SA * p.a_stage_bytes + p.SB * b_stage <= budget || p.T == 1) break;
   }
-  if (p.SA > kMaxSA) p.SA = kMaxSA;
   p.smem_bytes = p.SA * p.a_stage_bytes + p.SB * b_stage + tail + 1024;
   return p;
 }
@@ -597,7 +583,7 @@ inline int launch_halo_one(const CUtensorMap& tm0, const CUtensorMap& tm1, const
   int per_sm = 1;                                   // resident CTAs per SM (shared memory bound)
   if (2 * (smem_bytes + 1024) <= 227 * 1024 && 2 * HaloCfg<BN, T>::kTmemCols <= 512) per_sm = 2;
   const int grid = total < sm_count_cached() * per_sm ? total : sm_count_cached() * per_sm;
-  V2CE_CUDA_CHECK(launch_pdl(conv_halo_kernel<BN, T>, grid, kHaloThreads, (size_t)smem_bytes, s, tm0, tm1, a));
+  conv_halo_kernel<BN, T><<<grid, kHaloThreads, smem_bytes, s>>>(tm0, tm1, a);
   V2CE_LAUNCH_CHECK("conv_halo_kernel");
   return V2CE_OK;
 }

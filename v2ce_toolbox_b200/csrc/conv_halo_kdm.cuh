@@ -146,10 +146,8 @@ struct KdmInt { static constexpr int value = N; };
 // taps in the order the stride-2 variant multiplies them
 __device__ __constant__ int kS2TapOrder[9] = {4, 3, 5, 1, 7, 0, 2, 6, 8};
 
-// EW = epilogue warps: 8 (two per TMEM lane quarter, alternate slices) or, as an experiment switch, 16 (four per
-// quarter, every fourth slice; see launch_halo_kdm).
-template <bool SHORT, int T, int S, int EW = 8>
-__global__ void __launch_bounds__(128 + 32 * EW) conv_halo_kdm_kernel(const __grid_constant__ CUtensorMap tm0,
+template <bool SHORT, int T, int S>
+__global__ void __launch_bounds__(kKdmThreads) conv_halo_kdm_kernel(const __grid_constant__ CUtensorMap tm0,
                                                                      const __grid_constant__ CUtensorMap tm1,
                                                                      const __grid_constant__ ParityMaps pm,
                                                                      const HaloArgs a, const KdmShort sc) {
@@ -203,9 +201,6 @@ __global__ void __launch_bounds__(128 + 32 * EW) conv_halo_kdm_kernel(const __gr
   __syncthreads();
   tcgen05_fence_after();
   const uint32_t tmem_acc = *tmem_ptr;
-  // prologue done: let the next kernel of the stream be launched, then wait for the previous one's results
-  pdl_launch_dependents();
-  pdl_wait();
 
   // input slices a tile multiplies: d0-1 .. d0+T, minus the zero-padding slices -1 and D
   auto z_lo = [&](int d0) { return d0 > 0 ? d0 - 1 : 0; };
@@ -298,7 +293,7 @@ __global__ void __launch_bounds__(128 + 32 * EW) conv_halo_kdm_kernel(const __gr
       const uint32_t par_empty = (uint32_t)(((iter / G) & 1) ^ 1);
       const uint32_t acc_base = tmem_acc + (uint32_t)(slot0 * BN);
       for (int cc = 0; cc < ncc; ++cc) {
-        // zero-padded channels (64-channel pitch of a 32-channel tensor) are not multiplied
+        // channels beyond the real ones (the upper half of a 32-channel tensor's 64-channel rows) are not multiplied
         const int rem = (cc < a.ncc0) ? (a.real0 - cc * kBlockK) : (a.real1 - (cc - a.ncc0) * kBlockK);
         const int ks = rem >= kBlockK ? kBlockK / 16 : (rem + 15) / 16;
         const bool last_cc = (cc == ncc - 1);
@@ -435,8 +430,9 @@ __global__ void __launch_bounds__(128 + 32 * EW) conv_halo_kdm_kernel(const __gr
     }
   } else if (warp >= 4) {
     // ================= epilogue (warps 4-11) =================
+    constexpr int kEpiThreads = kKdmThreads - 128;
     const int quarter = warp & 3;                 // TMEM lane quarter this warp may read
-    constexpr int kParts = EW / 4;                // warps per lane quarter: they take the block's slices round robin
+    constexpr int kParts = kEpiThreads / 128;     // warps per lane quarter: they take the block's slices round robin
     const int half = (warp - 4) >> 2;             // which of them this warp is
     const int i = quarter * 32 + lane;            // accumulator row == TMEM lane
     const int th = i / a.PW, tw = i % a.PW;
@@ -448,8 +444,8 @@ __global__ void __launch_bounds__(128 + 32 * EW) conv_halo_kdm_kernel(const __gr
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++iter) {
       const TileCoord tc = decode_tile(tile, a, T, n_tiles);
       if (tc.n_tile != cur_n_tile) {              // (re)stage the folded BatchNorm scale/shift of this channel tile
-        asm volatile("bar.sync 1, %0;" ::"n"(32 * EW) : "memory");
-        for (int j = etid; j < BN; j += 32 * EW) {
+        asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
+        for (int j = etid; j < BN; j += kEpiThreads) {
           s_scale[j] = __ldg(a.scale + tc.n_tile * BN + j) * isg;
           s_shift[j] = __ldg(a.shift + tc.n_tile * BN + j);
           if (SHORT) {
@@ -457,7 +453,7 @@ __global__ void __launch_bounds__(128 + 32 * EW) conv_halo_kdm_kernel(const __gr
             s_shift2[j] = __ldg(sc.shift + tc.n_tile * BN + j);
           }
         }
-        asm volatile("bar.sync 1, %0;" ::"n"(32 * EW) : "memory");
+        asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
         cur_n_tile = tc.n_tile;
       }
       const int slot0 = (iter % G) * T;
@@ -645,18 +641,18 @@ inline int make_parity_map(CUtensorMap* map, const void* ptr, int B, int D, int 
   return V2CE_OK;
 }
 
-template <bool SHORT, int T, int S, int EW = 8>
+template <bool SHORT, int T, int S>
 inline int launch_kdm_one(const CUtensorMap& tm0, const CUtensorMap& tm1, const ParityMaps& pm, const HaloArgs& a,
                           const KdmShort& sc, int smem_bytes, cudaStream_t s) {
   static int configured[64] = {0};
   const int slot = device_slot();
   if (configured[slot] < smem_bytes) {
-    V2CE_CUDA_CHECK(cudaFuncSetAttribute(conv_halo_kdm_kernel<SHORT, T, S, EW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+    V2CE_CUDA_CHECK(cudaFuncSetAttribute(conv_halo_kdm_kernel<SHORT, T, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
     configured[slot] = smem_bytes;
   }
   const int total = a.B * (a.D / T) * a.tiles_h * a.tiles_w * (a.Cout / kKdmBN);
   const int grid = total < sm_count_cached() ? total : sm_count_cached();
-  V2CE_CUDA_CHECK(launch_pdl(conv_halo_kdm_kernel<SHORT, T, S, EW>, grid, 128 + 32 * EW, (size_t)smem_bytes, s, tm0, tm1, pm, a, sc));
+  conv_halo_kdm_kernel<SHORT, T, S><<<grid, kKdmThreads, smem_bytes, s>>>(tm0, tm1, pm, a, sc);
   V2CE_LAUNCH_CHECK("conv_halo_kdm_kernel");
   return V2CE_OK;
 }
@@ -665,13 +661,12 @@ inline int launch_kdm_one(const CUtensorMap& tm0, const CUtensorMap& tm1, const 
 // `pm` != nullptr: stride (1,2,2); a.H / a.W are the OUTPUT plane and pm the four parity views of the single source.
 inline int launch_halo_kdm(const CUtensorMap& tm0, const CUtensorMap& tm1, const HaloArgs& a, const KdmShort* sc, int smem_bytes,
                            cudaStream_t s, const ParityMaps* pm = nullptr) {
-  static const bool t8_only = getenv("V2CE_KDM_T8") && atoi(getenv("V2CE_KDM_T8"));
   if (a.D % kKdmT != 0 || a.Cout % kKdmBN != 0)
     return set_error(V2CE_ERR_INVALID, "depth-merged halo kernel: depth %d / Cout %d not supported", a.D, a.Cout);
   if (sc && (a.up_H > 0 || a.pred_w != nullptr || a.residual != nullptr))
     return set_error(V2CE_ERR_INVALID, "depth-merged halo kernel: the fused shortcut goes with a plain first conv");
   if (pm && a.ncc1 != 0) return set_error(V2CE_ERR_INVALID, "depth-merged halo kernel: stride 2 takes a single source");
-  const bool t16 = !sc && a.D % 16 == 0 && !t8_only;
+  const bool t16 = !sc && a.D % 16 == 0;
   HaloArgs b = a;
   b.T = t16 ? 16 : 8;
   const KdmShort none{nullptr, nullptr, nullptr, nullptr, 0};
@@ -682,12 +677,6 @@ inline int launch_halo_kdm(const CUtensorMap& tm0, const CUtensorMap& tm1, const
     return launch_kdm_one<false, 8, 2>(tm0, tm1, *pm, b, none, smem_bytes, s);
   }
   if (sc) return launch_kdm_one<true, 8, 1>(tm0, tm1, no_pm, b, *sc, smem_bytes, s);
-  // V2CE_KDM_EW16=1: 16 epilogue warps for the launches with few MMAs per slice (<= V2CE_KDM_EW16_MAXC channels, one
-  // chunk).  Measured on one box (profiles/layer_times_r2_h_*.txt) and left OFF: the head and decoders.3.conv2 do not get
-  // faster (0.470 / 0.540 ms against 0.458 / 0.530) and the whole power-capped forward gets 3 % slower (9.40 vs 9.07 ms).
-  static const bool ew16 = getenv("V2CE_KDM_EW16") && atoi(getenv("V2CE_KDM_EW16")) != 0;
-  static const int ew16_maxc = getenv("V2CE_KDM_EW16_MAXC") ? atoi(getenv("V2CE_KDM_EW16_MAXC")) : 32;
-  if (t16 && ew16 && a.ncc0 + a.ncc1 == 1 && a.real0 <= ew16_maxc) return launch_kdm_one<false, 16, 1, 16>(tm0, tm1, no_pm, b, none, smem_bytes, s);
   if (t16) return launch_kdm_one<false, 16, 1>(tm0, tm1, no_pm, b, none, smem_bytes, s);
   return launch_kdm_one<false, 8, 1>(tm0, tm1, no_pm, b, none, smem_bytes, s);
 }

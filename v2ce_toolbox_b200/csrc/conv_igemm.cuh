@@ -276,9 +276,6 @@ __global__ void __launch_bounds__(kThreads) conv_igemm_kernel(const ConvArgs a) 
   __syncthreads();
   tcgen05_fence_after();
   const uint32_t tmem_acc = *tmem_ptr;
-  // prologue done: let the next kernel of the stream be launched, then wait for the previous one's results
-  pdl_launch_dependents();
-  pdl_wait();
 
   if (warp < 8) {
     // ================= A producer (8 warps) =================
@@ -476,8 +473,8 @@ __global__ void __launch_bounds__(kThreads) conv_igemm_kernel(const ConvArgs a) 
 
 // Weight repack: fp32 (Cout, Cin_real, k,k,k) -> bf16 tiles [Cout/BN][num_kb][BN][64] with the 128B swizzle
 // applied per row (16-byte chunk q of row r is stored at chunk q ^ (r & 7)); k = tap*Cin_pad + p, zero padded.
-// Padded input channel p maps to a real channel through two segments (pad0/real0 | pad1/real1): activations
-// with fewer than 64 channels are stored with a 64-channel pitch so every TMA box is one 128-byte row.
+// Padded input channel p maps to a real channel through two segments (pad0/real0 | pad1/real1): the halo kernels
+// read activations with fewer than 64 channels as 64-channel rows so every TMA box row is 128 bytes.
 __global__ void pack_weights_kernel(const float* __restrict__ w, int Cout, int cin_real, int taps, int BN, int num_kb,
                                     int pad0, int real0, int pad1, int real1, __nv_bfloat16* __restrict__ out) {
   const int cin_pad = pad0 + pad1;
@@ -524,7 +521,7 @@ inline int launch_one(const ConvArgs& a, cudaStream_t s) {
   }
   const int m_tiles = (a.M + kBlockM - 1) / kBlockM;
   const int grid = m_tiles * (a.Cout / BN);
-  V2CE_CUDA_CHECK(launch_pdl(conv_igemm_kernel<BN, STAGES>, grid, kThreads, (size_t)L::kDynamicBytes, s, a));
+  conv_igemm_kernel<BN, STAGES><<<grid, kThreads, L::kDynamicBytes, s>>>(a);
   V2CE_LAUNCH_CHECK("conv_igemm_kernel");
   return V2CE_OK;
 }

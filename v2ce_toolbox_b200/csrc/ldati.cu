@@ -24,7 +24,6 @@
 #include "common.cuh"
 
 #include <limits.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace v2ce {
@@ -34,8 +33,6 @@ constexpr int kBins = 9;          // event bins per frame pair (10 voxel bins ->
 constexpr int kQ = 18;            // scanned quantities per plane: singles[9], multis[9]
 constexpr int kThreads = 256;
 constexpr int kKeyBias = 8;       // slack below the bin origin (ts may undershoot it by 1 us)
-constexpr int kTile = 2048;       // sort tile: 256 threads x 8 keys
-constexpr int kKeysPerThread = kTile / kThreads;
 // one-sweep sort (osw_*): 256 threads x 16 keys, <= 6-bit digits (64 digits = 32 counter lanes x 2 packed 16-bit counters)
 constexpr int kOswKpt = 16;
 constexpr int kOswTile = kThreads * kOswKpt;
@@ -483,43 +480,13 @@ __global__ void __launch_bounds__(kThreads) emit_kernel(const float* __restrict_
   const bool active = pix0 < P.HW;
   const float* plane0 = vox + ((size_t)(f * 2 + p) * 10) * P.HW;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  // ---- pass A: per-warp totals of the 18 quantities (singles / multi-event totals per bin) ----
+  // ---- per-warp totals of the 18 quantities (singles / multi-event totals per bin), left by the count pass ----
   __shared__ int wtot[kThreads / 32][kQ];
   __shared__ float2 s_par[kThreads / 32][32][V];      // (k, b) of every pixel of the block for the current bin
-  if (warp_partial != nullptr) {
-    // the count pass left this block's per-warp totals in its workspace: no second relocation pass over the voxels
-    if (threadIdx.x < (kThreads / 32) * kQ)
-      (&wtot[0][0])[threadIdx.x] =
-          warp_partial[(((size_t)f * 2 + p) * P.NB + blk) * ((kThreads / 32) * kQ) + threadIdx.x];
-  } else {
-    int tot[kQ];
-#pragma unroll
-    for (int q = 0; q < kQ; ++q) tot[q] = 0;
-    if (active) {
-      float y[V][10];
-      load_pixels<V>(plane0, P.HW, pix0, y);
-#pragma unroll
-      for (int v = 0; v < V; ++v) {
-        int n[kBins];
-        float tend[kBins];
-        relocate_any<BIDIR>(y[v], P.eps6, n, tend);
-#pragma unroll
-        for (int c = 0; c < kBins; ++c) {
-          tot[c] += (n[c] == 1);
-          tot[kBins + c] += (n[c] >= 2 && P.multi_events) ? n[c] : 0;
-        }
-      }
-    }
-#pragma unroll
-    for (int q = 0; q < kQ; ++q) {
-      int v = tot[q];
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-      if (lane == 0) wtot[warp][q] = v;
-    }
-  }
+  if (threadIdx.x < (kThreads / 32) * kQ)
+    (&wtot[0][0])[threadIdx.x] = warp_partial[(((size_t)f * 2 + p) * P.NB + blk) * ((kThreads / 32) * kQ) + threadIdx.x];
   __syncthreads();
-  // ---- pass B: bins in order, three-bin window of counts; voxels re-read (L1/L2 hits) ----
+  // ---- bins in order, three-bin window of counts; voxels re-read (L1/L2 hits) ----
   const int pol = 1 - p;                         // p-index 0 = positive plane -> polarity 1
   const int grp = (p == 1) ? 0 : 2;              // negative plane is emitted first
   const size_t bb = (((size_t)f * 2 + p) * P.NB + blk) * kQ;
@@ -770,48 +737,37 @@ __global__ void __launch_bounds__(kThreads) emit_kernel(const float* __restrict_
 }
 
 // ---------------------------------------------------------------------------------------
-// K6: segmented stable LSD radix sort on the key field.  Tiles never straddle segments.
+// K6: segmented stable LSD radix sort on the key field (one-sweep passes, osw_*).  Tiles never straddle segments.
 // ---------------------------------------------------------------------------------------
 struct SortWs {
   void* elem_a;
   void* elem_b;
-  int32_t* tile_first;   // [NS+1] first tile of each segment (exclusive scan of tiles per segment)
+  int32_t* tile_first;   // [NS+1] first 4096-key tile of each segment (exclusive scan of tiles per segment)
   int32_t* tile_seg;     // [NT_max]
-  int32_t* counts;       // [NT_max * radix]  (segment-major, digit-major, tile-minor)
-  int32_t* block_sums;   // scan scratch
-  // one-sweep path (osw_*): 4096-key tiles, per-segment digit histograms, decoupled look-back state
-  int32_t* tile_first4;  // [NS+1]
-  int32_t* tile_seg4;    // [NT4_max]
   char* osw_zero;        // start of the region cleared before every call: tickets, histograms, look-back state
   size_t osw_zero_bytes;
   int32_t* tickets;      // [kOswMaxPasses]
   int32_t* seg_hist;     // [kOswMaxPasses][NS][64]
-  unsigned long long* tstate;   // [kOswMaxPasses][NT4_max][64]
+  unsigned long long* tstate;   // [kOswMaxPasses][NT_max][64]
   int32_t* chunk_seg;    // [ceil(total / 128)] segment of the first record of every 128-record pack chunk
   size_t bytes;
   int nt_max;
-  int nt4_max;
 };
 
 static SortWs carve_sort_ws(void* ws, const Geometry& g, int64_t total, int elem_bytes) {
   Arena a(ws, (size_t)-1);
   SortWs s;
   const int ns = g.F * kBins;
-  s.nt_max = (int)((total + kTile - 1) / kTile) + ns;
   s.elem_a = a.take<char>((size_t)(total > 0 ? total : 1) * elem_bytes);
   s.elem_b = a.take<char>((size_t)(total > 0 ? total : 1) * elem_bytes);
+  s.nt_max = (int)((total + kOswTile - 1) / kOswTile) + ns;
   s.tile_first = a.take<int32_t>((size_t)ns + 1);
   s.tile_seg = a.take<int32_t>((size_t)s.nt_max);
-  s.counts = a.take<int32_t>((size_t)s.nt_max * 256 + 1);
-  s.block_sums = a.take<int32_t>((size_t)s.nt_max * 256 / 1024 + 2);
-  s.nt4_max = (int)((total + kOswTile - 1) / kOswTile) + ns;
-  s.tile_first4 = a.take<int32_t>((size_t)ns + 1);
-  s.tile_seg4 = a.take<int32_t>((size_t)s.nt4_max);
   const int passes = osw_passes(g.key_bits);
   s.tickets = a.take<int32_t>(kOswMaxPasses);
   s.osw_zero = reinterpret_cast<char*>(s.tickets);
   s.seg_hist = a.take<int32_t>((size_t)passes * ns * kOswRadix);
-  s.tstate = a.take<unsigned long long>((size_t)passes * s.nt4_max * kOswRadix);
+  s.tstate = a.take<unsigned long long>((size_t)passes * s.nt_max * kOswRadix);
   s.osw_zero_bytes = (size_t)((a.base + a.off) - s.osw_zero);
   s.chunk_seg = a.take<int32_t>((size_t)(total / kPackRecsPerWarpDecl) + 2);
   s.bytes = align_up(a.off, 256);
@@ -859,252 +815,11 @@ __global__ void fill_tile_seg_kernel(const int32_t* __restrict__ tile_first, int
   tile_seg[t] = lo;
 }
 
-template <typename Elem>
-__global__ void __launch_bounds__(kThreads) sort_hist_kernel(const Elem* __restrict__ in,
-                                                              const int64_t* __restrict__ seg_start,
-                                                              const int32_t* __restrict__ tile_first,
-                                                              const int32_t* __restrict__ tile_seg, int ns, int shift,
-                                                              int radix_bits, int32_t* __restrict__ counts) {
-  const int tile = blockIdx.x;
-  if (tile >= tile_first[ns]) return;
-  const int seg = tile_seg[tile];
-  const int tin = tile - tile_first[seg];
-  const int ntile_seg = tile_first[seg + 1] - tile_first[seg];
-  const long long start = seg_start[seg] + (long long)tin * kTile;
-  const int cnt = (int)min((long long)kTile, seg_start[seg + 1] - start);
-  const int radix = 1 << radix_bits;
-  __shared__ int hist[256];
-  for (int i = threadIdx.x; i < radix; i += kThreads) hist[i] = 0;
-  __syncthreads();
-  for (int i = threadIdx.x; i < cnt; i += kThreads) {
-    const unsigned d = (unsigned)(in[start + i] >> shift) & (radix - 1);
-    atomicAdd(&hist[d], 1);
-  }
-  __syncthreads();
-  // layout: [segment][digit][tile in segment]; segment block starts at radix * tile_first[seg]
-  int32_t* dst = counts + (size_t)radix * tile_first[seg];
-  for (int d = threadIdx.x; d < radix; d += kThreads) dst[(size_t)d * ntile_seg + tin] = hist[d];
-}
-
-// generic int32 exclusive scan, three phases (n up to ~10^8)
-__global__ void scan_reduce_kernel(const int32_t* __restrict__ in, int n, int32_t* __restrict__ block_sums) {
-  const int base = blockIdx.x * 1024;
-  int v = 0;
-  for (int i = threadIdx.x; i < 1024; i += blockDim.x)
-    if (base + i < n) v += in[base + i];
-  __shared__ int red[32];
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int s = 0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += red[w];
-    block_sums[blockIdx.x] = s;
-  }
-}
-
-__global__ void scan_block_sums_kernel(int32_t* __restrict__ block_sums, int nb) {
-  // single block, sequential chunks of blockDim.x
-  __shared__ int carry_s;
-  __shared__ int wsum[32];
-  if (threadIdx.x == 0) carry_s = 0;
-  __syncthreads();
-  for (int base = 0; base < nb; base += blockDim.x) {
-    const int i = base + threadIdx.x;
-    const int v = (i < nb) ? block_sums[i] : 0;
-    int inc = warp_incl_scan(v);
-    if ((threadIdx.x & 31) == 31) wsum[threadIdx.x >> 5] = inc;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-      int w = (threadIdx.x < (blockDim.x >> 5)) ? wsum[threadIdx.x] : 0;
-      int wi = warp_incl_scan(w);
-      wsum[threadIdx.x] = wi - w;
-    }
-    __syncthreads();
-    const int ex = carry_s + wsum[threadIdx.x >> 5] + inc - v;
-    if (i < nb) block_sums[i] = ex;
-    __syncthreads();
-    if (threadIdx.x == blockDim.x - 1) carry_s = ex + v;
-    __syncthreads();
-  }
-}
-
-__global__ void __launch_bounds__(256) scan_apply_kernel(int32_t* __restrict__ data, int n,
-                                                          const int32_t* __restrict__ block_sums) {
-  // each block scans 1024 values: 256 threads x 4 consecutive
-  const int base = blockIdx.x * 1024 + threadIdx.x * 4;
-  int v[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) v[i] = (base + i < n) ? data[base + i] : 0;
-  const int tsum = v[0] + v[1] + v[2] + v[3];
-  int inc = warp_incl_scan(tsum);
-  __shared__ int wsum[8];
-  if ((threadIdx.x & 31) == 31) wsum[threadIdx.x >> 5] = inc;
-  __syncthreads();
-  int woff = 0;
-  for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) woff += wsum[w];
-  int run = block_sums[blockIdx.x] + woff + inc - tsum;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    if (base + i < n) data[base + i] = run;
-    run += v[i];
-  }
-}
-
-// STAGED: the tile is first ordered by digit in shared memory (same stable rank), then written out run by run, so
-// consecutive threads store consecutive addresses of a digit's run; unstaged, every lane stores to its own digit's
-// position (one 32-byte sector per 4-byte key).
-template <typename Elem, bool STAGED>
-__global__ void __launch_bounds__(kThreads) sort_scatter_kernel(const Elem* __restrict__ in, Elem* __restrict__ out,
-                                                                 const int64_t* __restrict__ seg_start,
-                                                                 const int32_t* __restrict__ tile_first,
-                                                                 const int32_t* __restrict__ tile_seg, int ns, int shift,
-                                                                 int radix_bits, const int32_t* __restrict__ scanned) {
-  const int tile = blockIdx.x;
-  if (tile >= tile_first[ns]) return;
-  const int seg = tile_seg[tile];
-  const int tin = tile - tile_first[seg];
-  const int ntile_seg = tile_first[seg + 1] - tile_first[seg];
-  const long long start = seg_start[seg] + (long long)tin * kTile;
-  const int cnt = (int)min((long long)kTile, seg_start[seg + 1] - start);
-  const int radix = 1 << radix_bits;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  constexpr int kWarps = kThreads / 32;
-  __shared__ int wcnt[kWarps][256];     // per-warp digit counters -> exclusive bases
-  __shared__ int gbase[256];            // global position of this tile's first key of each digit
-  for (int i = threadIdx.x; i < kWarps * 256; i += kThreads) (&wcnt[0][0])[i] = 0;
-  __syncthreads();
-  // warp w owns keys [w*256, w*256+256) of the tile, 8 rounds of 32 consecutive keys:
-  // memory order == (warp, round, lane), which is what keeps the pass stable.
-  Elem key[kKeysPerThread];
-  int rank[kKeysPerThread];
-  unsigned dig[kKeysPerThread];
-#pragma unroll
-  for (int r = 0; r < kKeysPerThread; ++r) {
-    const int i = warp * (kTile / kWarps) + r * 32 + lane;
-    const bool valid = i < cnt;
-    key[r] = valid ? in[start + i] : (Elem)0;
-    const unsigned d = valid ? ((unsigned)(key[r] >> shift) & (radix - 1)) : 0xFFFFu;
-    dig[r] = d;
-    const unsigned peers = __match_any_sync(0xffffffffu, d);
-    const int leader = __ffs(peers) - 1;
-    const int before = __popc(peers & ((1u << lane) - 1u));
-    int old = 0;
-    if (valid && lane == leader) {
-      old = wcnt[warp][d];
-      wcnt[warp][d] = old + __popc(peers);
-    }
-    old = __shfl_sync(0xffffffffu, old, leader);
-    rank[r] = old + before;
-    __syncwarp();
-  }
-  __syncthreads();
-  // exclusive prefix over warps per digit; fetch the scanned global base of (seg, digit, tile)
-  int digit_total = 0;                  // radix <= kThreads: thread d owns digit d
-  for (int d = threadIdx.x; d < radix; d += kThreads) {
-    int run = 0;
-#pragma unroll
-    for (int w = 0; w < kWarps; ++w) {
-      const int c = wcnt[w][d];
-      wcnt[w][d] = run;
-      run += c;
-    }
-    digit_total = run;
-    gbase[d] = scanned[(size_t)radix * tile_first[seg] + (size_t)d * ntile_seg + tin];
-  }
-  if (!STAGED) {
-    __syncthreads();
-#pragma unroll
-    for (int r = 0; r < kKeysPerThread; ++r) {
-      if (dig[r] != 0xFFFFu) out[(size_t)gbase[dig[r]] + wcnt[warp][dig[r]] + rank[r]] = key[r];
-    }
-  } else {
-    __shared__ int lbase[256];          // tile-local position of each digit's first key
-    __shared__ int wsum[kWarps];
-    __shared__ Elem stage[kTile];
-    const int inc = warp_incl_scan(digit_total);
-    if (lane == 31) wsum[warp] = inc;
-    __syncthreads();
-    int woff = 0;
-    for (int w = 0; w < warp; ++w) woff += wsum[w];
-    if ((int)threadIdx.x < radix) lbase[threadIdx.x] = woff + inc - digit_total;
-    __syncthreads();
-#pragma unroll
-    for (int r = 0; r < kKeysPerThread; ++r) {
-      if (dig[r] != 0xFFFFu) stage[lbase[dig[r]] + wcnt[warp][dig[r]] + rank[r]] = key[r];
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < cnt; i += kThreads) {
-      const Elem k = stage[i];
-      const unsigned d = (unsigned)(k >> shift) & (radix - 1);
-      out[(size_t)gbase[d] + (i - lbase[d])] = k;
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------
-// K7: pack sorted elements into 13-byte records, staged through shared memory so the
-// byte stream leaves the SM as aligned 16-byte stores.
-// ---------------------------------------------------------------------------------------
-template <typename Elem>
-__global__ void __launch_bounds__(kThreads) pack_kernel(const Elem* __restrict__ in, const int64_t* __restrict__ seg_start,
-                                                         const int32_t* __restrict__ tile_first,
-                                                         const int32_t* __restrict__ tile_seg, int ns, DevParams P,
-                                                         const int64_t* __restrict__ frame_offset_us,
-                                                         uint8_t* __restrict__ out) {
-  const int tile = blockIdx.x;
-  if (tile >= tile_first[ns]) return;
-  const int seg = tile_seg[tile];
-  const int tin = tile - tile_first[seg];
-  const long long start = seg_start[seg] + (long long)tin * kTile;
-  const int cnt = (int)min((long long)kTile, seg_start[seg + 1] - start);
-  const int f = seg / kBins, c = seg % kBins;
-  long long base_ts = P.bin_base[c] - kKeyBias;
-  long long off = 0;
-  if (P.add_frame_offset && frame_offset_us != nullptr) off = frame_offset_us[f];
-  __shared__ __align__(16) uint8_t stage[kTile * 13 + 32];
-  const unsigned long long gbyte = (unsigned long long)start * 13ull;
-  const unsigned long long gaddr = (unsigned long long)(uintptr_t)out + gbyte;
-  const int mis = (int)(gaddr & 15ull);        // stage[mis + k] <-> out[gbyte + k]
-  const unsigned long long pix_mask = (1ull << P.pix_bits) - 1ull;
-  for (int i = threadIdx.x; i < cnt; i += kThreads) {
-    const unsigned long long e = (unsigned long long)in[start + i];
-    const int pix = (int)(e & pix_mask);
-    const int pol = (int)((e >> P.pix_bits) & 1ull);
-    const long long key = (long long)(e >> (P.pix_bits + 1));
-    long long ts = (key == 0) ? P.nan_ts : (base_ts + key);
-    ts = (long long)((unsigned long long)ts + (unsigned long long)off);
-    const short x = (short)(pix % P.W), y = (short)(pix / P.W);
-    uint8_t* d = stage + mis + i * 13;
-#pragma unroll
-    for (int b = 0; b < 8; ++b) d[b] = (uint8_t)((unsigned long long)ts >> (8 * b));
-    d[8] = (uint8_t)(x & 0xff);  d[9] = (uint8_t)((x >> 8) & 0xff);
-    d[10] = (uint8_t)(y & 0xff); d[11] = (uint8_t)((y >> 8) & 0xff);
-    d[12] = (uint8_t)pol;
-  }
-  __syncthreads();
-  const int nbytes = cnt * 13;
-  const int lo = mis, hi = mis + nbytes;              // valid byte range inside stage
-  uint8_t* gout = out + gbyte - mis;                  // 16-byte aligned
-  const int nvec = (hi + 15) / 16;
-  for (int v = threadIdx.x; v < nvec; v += kThreads) {
-    const int b0 = v * 16;
-    if (b0 >= lo && b0 + 16 <= hi) {
-      *reinterpret_cast<uint4*>(gout + b0) = *reinterpret_cast<const uint4*>(stage + b0);
-    } else {
-      for (int b = max(b0, lo); b < min(b0 + 16, hi); ++b) gout[b] = stage[b];
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------
-// K6': one-sweep segmented stable LSD radix sort (the default path).
-//
-// ncu on the first-generation scatter (profiles/ncu_ldati_r2_a.txt): 88 % of the ADU pipe -- eight dependent
-// __match_any_sync rounds per thread rank the keys -- at 1.4 instructions per cycle per SM, 140 us per pass for
-// 21.6 M keys, plus a histogram kernel, three scan kernels and a second read of every key per pass.  Here a pass is
-// ONE kernel over 4096-key tiles:
+// K6 passes.  A histogram / scan / scatter sort on 2048-key tiles spent 140 us per pass for 21.6 M keys in its
+// scatter alone (88 % of the ADU pipe: eight dependent __match_any_sync rounds per thread rank the keys;
+// profiles/ncu_ldati_r2_a.txt), plus a histogram kernel, three scan kernels and a second read of every key per pass.
+// Here a pass is ONE kernel over 4096-key tiles:
 //   * the tile's digit counts are chained to the tiles before it IN ITS SEGMENT by decoupled look-back (one 64-bit
 //     status word per (tile, digit): flag | count); tiles take tickets from an atomic counter, so a tile only ever
 //     waits for tiles that already run;
@@ -1323,12 +1038,12 @@ __global__ void __launch_bounds__(kThreads, 4) osw_scatter_kernel(const Elem* __
 }
 
 // ---------------------------------------------------------------------------------------
-// K7': 13-byte records, linear over the whole sorted stream.  FOUR consecutive records are exactly 13 aligned 32-bit
+// K7: 13-byte records, linear over the whole sorted stream.  FOUR consecutive records are exactly 13 aligned 32-bit
 // words, so a thread loads four elements with one 16-byte load, builds their 13 words in registers with fixed byte
 // permutes, and the warp transposes its 32 x 13 words through shared memory (stride 13: conflict free) into 416
-// consecutive words that leave as 16-byte coalesced stores.  No byte stores anywhere.  The first generation staged
-// bytes through shared memory with 13 one-byte stores per record (92 % of the LSU wavefront peak, 103 us for 21.6 M
-// events); assembling the words with 5 shuffles each was worse (230 us, 311 instructions per 32 records --
+// consecutive words that leave as 16-byte coalesced stores.  No byte stores anywhere.  Staging bytes through shared
+// memory with 13 one-byte stores per record reached 92 % of the LSU wavefront peak and took 103 us for 21.6 M
+// events; assembling the words with 5 shuffles each was worse (230 us, 311 instructions per 32 records --
 // profiles/ncu_ldati_r2_c.txt).  A record's segment (bin origin, frame offset) is found from a per-128-record table.
 // ---------------------------------------------------------------------------------------
 constexpr int kPackRecsPerWarp = kPackRecsPerWarpDecl;
@@ -1780,22 +1495,42 @@ extern "C" int v2ce_ldati_count_ef(const float* voxels_dev, const v2ce_ldati_par
   return V2CE_OK;
 }
 
-// Kernel variants, read per call so one process can compare them (tests/test_gpu_ldati.py, tools/ldati_bench.py);
-// both default ON: bit-exact in all four combinations, 1-4 % faster together on the microbench
-// (profiles/ldati_variants_r1.json).  Set to 0 to get the first-generation path.
-//   V2CE_LDATI_REUSE_WARP_TOTALS  the emit pass reads the per-warp totals the count pass stored instead of
-//                                 relocating every pixel a second time to rebuild them
-//   V2CE_LDATI_STAGED_SCATTER     every sort tile is ordered by digit in shared memory before the scatter
-//                                 (see sort_scatter_kernel)
-static bool env_flag(const char* name, bool dflt) {
-  const char* v = getenv(name);
-  return (v && *v) ? atoi(v) != 0 : dflt;
+// Sorts the `total` elements in sw.elem_a stably by their key field inside each of the `ns` segments
+// [seg_start[i], seg_start[i+1]) and writes their 13-byte records to `out`.  P supplies the field widths and the
+// timestamp origin of every segment (see pack_linear_kernel).
+template <typename Elem>
+static int sort_and_pack(const SortWs& sw, const int64_t* seg_start, int ns, int64_t total, const DevParams& P,
+                         const int64_t* frame_off, uint8_t* out, cudaStream_t s) {
+  // one-sweep LSD passes over the key field, <= 6 bits each
+  const int passes = osw_passes(P.key_bits);
+  const int rb = (P.key_bits + passes - 1) / passes;
+  build_tiles_kernel<<<1, 1024, 0, s>>>(seg_start, ns, kOswTile, sw.tile_first);
+  V2CE_LAUNCH_CHECK("ldati::build_tiles_kernel");
+  fill_tile_seg_kernel<<<(sw.nt_max + 255) / 256, 256, 0, s>>>(sw.tile_first, ns, sw.tile_seg);
+  V2CE_LAUNCH_CHECK("ldati::fill_tile_seg_kernel");
+  V2CE_CUDA_CHECK(cudaMemsetAsync(sw.osw_zero, 0, sw.osw_zero_bytes, s));
+  Elem* src = static_cast<Elem*>(sw.elem_a);
+  Elem* dst = static_cast<Elem*>(sw.elem_b);
+  osw_hist_kernel<Elem><<<sw.nt_max, kThreads, 0, s>>>(src, seg_start, sw.tile_first, sw.tile_seg, ns, P.pix_bits + 1, rb,
+                                                       passes, sw.seg_hist);
+  V2CE_LAUNCH_CHECK("ldati::osw_hist_kernel");
+  const size_t smem = (size_t)kOswCounterWords * 4 > (size_t)kOswStageSlots * sizeof(Elem)
+                          ? (size_t)kOswCounterWords * 4 : (size_t)kOswStageSlots * sizeof(Elem);
+  for (int pass = 0; pass < passes; ++pass) {
+    osw_scatter_kernel<Elem><<<sw.nt_max, kThreads, smem, s>>>(
+        src, dst, seg_start, sw.tile_first, sw.tile_seg, ns, P.pix_bits + 1 + pass * rb, rb,
+        sw.seg_hist + (size_t)pass * ns * kOswRadix, sw.tstate + (size_t)pass * sw.nt_max * kOswRadix, sw.tickets + pass);
+    V2CE_LAUNCH_CHECK("ldati::osw_scatter_kernel");
+    Elem* t = src; src = dst; dst = t;
+  }
+  const long long nchunks = (total + kPackRecsPerWarp - 1) / kPackRecsPerWarp;
+  pack_chunk_seg_kernel<<<(int)((nchunks + 255) / 256), 256, 0, s>>>(seg_start, ns, total, sw.chunk_seg);
+  V2CE_LAUNCH_CHECK("ldati::pack_chunk_seg_kernel");
+  pack_linear_kernel<Elem><<<(int)((nchunks + kThreads / 32 - 1) / (kThreads / 32)), kThreads, 0, s>>>(
+      src, seg_start, sw.chunk_seg, ns, total, P, frame_off, out);
+  V2CE_LAUNCH_CHECK("ldati::pack_linear_kernel");
+  return V2CE_OK;
 }
-static bool reuse_warp_totals() { return env_flag("V2CE_LDATI_REUSE_WARP_TOTALS", true); }
-static bool staged_scatter() { return env_flag("V2CE_LDATI_STAGED_SCATTER", true); }
-//   V2CE_LDATI_ONESWEEP           1 (default): one-sweep sort passes (osw_* kernels); 0: the first-generation
-//                                 histogram / scan / scatter passes on 2048-key tiles
-static bool onesweep() { return env_flag("V2CE_LDATI_ONESWEEP", true); }
 
 template <typename Elem>
 static int emit_impl(const float* vox, const v2ce_ldati_params* p, const Geometry& g, const CountWs& cw, void* emit_ws,
@@ -1806,15 +1541,12 @@ static int emit_impl(const float* vox, const v2ce_ldati_params* p, const Geometr
     return set_error(V2CE_ERR_WORKSPACE, "emit workspace too small: need %zu, got %zu", sw.bytes, emit_ws_bytes);
   DevParams P = make_dev_params(p, g);
   P.draws_m = draws_m;
-  const int ns = g.F * kBins;
   Elem* ea = static_cast<Elem*>(sw.elem_a);
-  Elem* eb = static_cast<Elem*>(sw.elem_b);
   V2CE_CUDA_CHECK(cudaMemsetAsync(status, 0, 4 * sizeof(int32_t), s));
   dim3 grid(g.NB, 2, g.F);
-  const int32_t* wp = reuse_warp_totals() ? cw.warp_partial : nullptr;
 #define V2CE_LAUNCH_EMIT(V_, BIDIR_, POOL_)                                                                      \
   emit_kernel<V_, Elem, BIDIR_, POOL_><<<grid, kThreads, 0, s>>>(vox, P, cw.block_base, cw.group_base, cw.seg_start, \
-                                                                  wp, cw.counts_all, draws, ea, status)
+                                                                  cw.warp_partial, cw.counts_all, draws, ea, status)
   const bool bidir = p->bidirectional != 0, pool = g.pooling != 0;
   if (g.V == 4) {
     if (bidir) { if (pool) V2CE_LAUNCH_EMIT(4, true, true); else V2CE_LAUNCH_EMIT(4, true, false); }
@@ -1826,73 +1558,7 @@ static int emit_impl(const float* vox, const v2ce_ldati_params* p, const Geometr
 #undef V2CE_LAUNCH_EMIT
   V2CE_LAUNCH_CHECK("ldati::emit_kernel");
   if (total == 0) return V2CE_OK;
-  Elem* src = ea;
-  Elem* dst = eb;
-  const bool osw = onesweep();
-  if (!osw) {
-    build_tiles_kernel<<<1, 1024, 0, s>>>(cw.seg_start, ns, kTile, sw.tile_first);
-    V2CE_LAUNCH_CHECK("ldati::build_tiles_kernel");
-    fill_tile_seg_kernel<<<(sw.nt_max + 255) / 256, 256, 0, s>>>(sw.tile_first, ns, sw.tile_seg);
-    V2CE_LAUNCH_CHECK("ldati::fill_tile_seg_kernel");
-  }
-  if (osw) {
-    // one-sweep LSD passes over the key field, <= 6 bits each
-    const int passes = osw_passes(g.key_bits);
-    const int rb = (g.key_bits + passes - 1) / passes;
-    build_tiles_kernel<<<1, 1024, 0, s>>>(cw.seg_start, ns, kOswTile, sw.tile_first4);
-    V2CE_LAUNCH_CHECK("ldati::build_tiles_kernel");
-    fill_tile_seg_kernel<<<(sw.nt4_max + 255) / 256, 256, 0, s>>>(sw.tile_first4, ns, sw.tile_seg4);
-    V2CE_LAUNCH_CHECK("ldati::fill_tile_seg_kernel");
-    V2CE_CUDA_CHECK(cudaMemsetAsync(sw.osw_zero, 0, sw.osw_zero_bytes, s));
-    osw_hist_kernel<Elem><<<sw.nt4_max, kThreads, 0, s>>>(src, cw.seg_start, sw.tile_first4, sw.tile_seg4, ns, g.pix_bits + 1, rb,
-                                                          passes, sw.seg_hist);
-    V2CE_LAUNCH_CHECK("ldati::osw_hist_kernel");
-    const size_t smem = (size_t)kOswCounterWords * 4 > (size_t)kOswStageSlots * sizeof(Elem)
-                            ? (size_t)kOswCounterWords * 4 : (size_t)kOswStageSlots * sizeof(Elem);
-    for (int pass = 0; pass < passes; ++pass) {
-      osw_scatter_kernel<Elem><<<sw.nt4_max, kThreads, smem, s>>>(
-          src, dst, cw.seg_start, sw.tile_first4, sw.tile_seg4, ns, g.pix_bits + 1 + pass * rb, rb,
-          sw.seg_hist + (size_t)pass * ns * kOswRadix, sw.tstate + (size_t)pass * sw.nt4_max * kOswRadix, sw.tickets + pass);
-      V2CE_LAUNCH_CHECK("ldati::osw_scatter_kernel");
-      Elem* t = src; src = dst; dst = t;
-    }
-    const long long nchunks = (total + kPackRecsPerWarp - 1) / kPackRecsPerWarp;
-    pack_chunk_seg_kernel<<<(int)((nchunks + 255) / 256), 256, 0, s>>>(cw.seg_start, ns, total, sw.chunk_seg);
-    V2CE_LAUNCH_CHECK("ldati::pack_chunk_seg_kernel");
-    pack_linear_kernel<Elem><<<(int)((nchunks + kThreads / 32 - 1) / (kThreads / 32)), kThreads, 0, s>>>(
-        src, cw.seg_start, sw.chunk_seg, ns, total, P, frame_off, out);
-    V2CE_LAUNCH_CHECK("ldati::pack_linear_kernel");
-    return V2CE_OK;
-  }
-  // first-generation path: LSD passes over the key field, <= 8 bits each
-  const int passes = osw ? 0 : (g.key_bits + 7) / 8;
-  const int rb = osw ? 0 : (g.key_bits + passes - 1) / passes;
-  for (int pass = 0; pass < passes; ++pass) {
-    const int shift = g.pix_bits + 1 + pass * rb;
-    const int radix = 1 << rb;
-    const int ncounts = sw.nt_max * radix;
-    sort_hist_kernel<Elem><<<sw.nt_max, kThreads, 0, s>>>(src, cw.seg_start, sw.tile_first, sw.tile_seg, ns, shift, rb,
-                                                          sw.counts);
-    V2CE_LAUNCH_CHECK("ldati::sort_hist_kernel");
-    const int nblk = (ncounts + 1023) / 1024;
-    scan_reduce_kernel<<<nblk, 256, 0, s>>>(sw.counts, ncounts, sw.block_sums);
-    V2CE_LAUNCH_CHECK("ldati::scan_reduce_kernel");
-    scan_block_sums_kernel<<<1, 1024, 0, s>>>(sw.block_sums, nblk);
-    V2CE_LAUNCH_CHECK("ldati::scan_block_sums_kernel");
-    scan_apply_kernel<<<nblk, 256, 0, s>>>(sw.counts, ncounts, sw.block_sums);
-    V2CE_LAUNCH_CHECK("ldati::scan_apply_kernel");
-    if (staged_scatter())
-      sort_scatter_kernel<Elem, true><<<sw.nt_max, kThreads, 0, s>>>(src, dst, cw.seg_start, sw.tile_first, sw.tile_seg,
-                                                                     ns, shift, rb, sw.counts);
-    else
-      sort_scatter_kernel<Elem, false><<<sw.nt_max, kThreads, 0, s>>>(src, dst, cw.seg_start, sw.tile_first, sw.tile_seg,
-                                                                      ns, shift, rb, sw.counts);
-    V2CE_LAUNCH_CHECK("ldati::sort_scatter_kernel");
-    Elem* t = src; src = dst; dst = t;
-  }
-  pack_kernel<Elem><<<sw.nt_max, kThreads, 0, s>>>(src, cw.seg_start, sw.tile_first, sw.tile_seg, ns, P, frame_off, out);
-  V2CE_LAUNCH_CHECK("ldati::pack_kernel");
-  return V2CE_OK;
+  return sort_and_pack<Elem>(sw, cw.seg_start, g.F * kBins, total, P, frame_off, out, s);
 }
 
 extern "C" int v2ce_ldati_emit(const float* voxels_dev, const v2ce_ldati_params* p, const void* count_ws_dev,
@@ -1996,35 +1662,13 @@ extern "C" int v2ce_baseline_emit(const float* voxels_dev, const v2ce_baseline_p
     return set_error(V2CE_ERR_WORKSPACE, "emit workspace too small: need %zu, got %zu", sw.bytes, emit_ws_bytes);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const BaseDev P = base_dev(p, bg);
-  Elem* src = static_cast<Elem*>(sw.elem_a);
-  Elem* dst = static_cast<Elem*>(sw.elem_b);
   V2CE_CUDA_CHECK(cudaMemsetAsync(status_dev, 0, 4 * sizeof(int32_t), s));
   if (total_events == 0) return V2CE_OK;
+  Elem* elems = static_cast<Elem*>(sw.elem_a);
   dim3 grid(bg.NB, 2, p->n_frames);
-  if (bg.V == 4) base_emit_kernel<4><<<grid, kThreads, 0, s>>>(voxels_dev, P, cw.block_base, cw.group_base, cw.seg_start, src, status_dev);
-  else base_emit_kernel<1><<<grid, kThreads, 0, s>>>(voxels_dev, P, cw.block_base, cw.group_base, cw.seg_start, src, status_dev);
+  if (bg.V == 4) base_emit_kernel<4><<<grid, kThreads, 0, s>>>(voxels_dev, P, cw.block_base, cw.group_base, cw.seg_start, elems, status_dev);
+  else base_emit_kernel<1><<<grid, kThreads, 0, s>>>(voxels_dev, P, cw.block_base, cw.group_base, cw.seg_start, elems, status_dev);
   V2CE_LAUNCH_CHECK("ldati::base_emit_kernel");
-  // one sort segment per frame
-  const int ns = p->n_frames;
-  const int passes = osw_passes(g.key_bits);
-  const int rb = (g.key_bits + passes - 1) / passes;
-  build_tiles_kernel<<<1, 1024, 0, s>>>(cw.seg_start, ns, kOswTile, sw.tile_first4);
-  V2CE_LAUNCH_CHECK("ldati::build_tiles_kernel");
-  fill_tile_seg_kernel<<<(sw.nt4_max + 255) / 256, 256, 0, s>>>(sw.tile_first4, ns, sw.tile_seg4);
-  V2CE_LAUNCH_CHECK("ldati::fill_tile_seg_kernel");
-  V2CE_CUDA_CHECK(cudaMemsetAsync(sw.osw_zero, 0, sw.osw_zero_bytes, s));
-  osw_hist_kernel<Elem><<<sw.nt4_max, kThreads, 0, s>>>(src, cw.seg_start, sw.tile_first4, sw.tile_seg4, ns, g.pix_bits + 1, rb, passes,
-                                                        sw.seg_hist);
-  V2CE_LAUNCH_CHECK("ldati::osw_hist_kernel");
-  const size_t smem = (size_t)kOswCounterWords * 4 > (size_t)kOswStageSlots * sizeof(Elem) ? (size_t)kOswCounterWords * 4
-                                                                                           : (size_t)kOswStageSlots * sizeof(Elem);
-  for (int pass = 0; pass < passes; ++pass) {
-    osw_scatter_kernel<Elem><<<sw.nt4_max, kThreads, smem, s>>>(src, dst, cw.seg_start, sw.tile_first4, sw.tile_seg4, ns,
-                                                                g.pix_bits + 1 + pass * rb, rb, sw.seg_hist + (size_t)pass * ns * kOswRadix,
-                                                                sw.tstate + (size_t)pass * sw.nt4_max * kOswRadix, sw.tickets + pass);
-    V2CE_LAUNCH_CHECK("ldati::osw_scatter_kernel");
-    Elem* t = src; src = dst; dst = t;
-  }
   // records: the LDATI record writer with one segment per frame whose key origin is the frame's
   DevParams D;
   memset(&D, 0, sizeof(D));
@@ -2034,11 +1678,5 @@ extern "C" int v2ce_baseline_emit(const float* voxels_dev, const v2ce_baseline_p
   D.nan_ts = LLONG_MIN;
   D.segs_per_frame = 1;
   D.bin_base[0] = p->key_base_us;
-  const long long nchunks = (total_events + kPackRecsPerWarp - 1) / kPackRecsPerWarp;
-  pack_chunk_seg_kernel<<<(int)((nchunks + 255) / 256), 256, 0, s>>>(cw.seg_start, ns, total_events, sw.chunk_seg);
-  V2CE_LAUNCH_CHECK("ldati::pack_chunk_seg_kernel");
-  pack_linear_kernel<Elem><<<(int)((nchunks + kThreads / 32 - 1) / (kThreads / 32)), kThreads, 0, s>>>(
-      src, cw.seg_start, sw.chunk_seg, ns, total_events, D, frame_offset_us_dev, events_out_dev);
-  V2CE_LAUNCH_CHECK("ldati::pack_linear_kernel");
-  return V2CE_OK;
+  return sort_and_pack<Elem>(sw, cw.seg_start, p->n_frames, total_events, D, frame_offset_us_dev, events_out_dev, s);
 }

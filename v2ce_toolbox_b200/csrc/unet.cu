@@ -76,7 +76,7 @@ static const LayerSpec kLayers[] = {
 constexpr int kNumLayers = sizeof(kLayers) / sizeof(kLayers[0]);
 
 // ------------------------------------------------------------------------------------------
-// head: Conv3d(2->32, k3, p1, bias) + LeakyReLU(0.01), fp32 in (B,L,2,H,W) -> bf16 NDHWC (pitch 64)
+// head: Conv3d(2->32, k3, p1, bias) + LeakyReLU(0.01), fp32 in (B,L,2,H,W) -> bf16 NDHWC
 // ------------------------------------------------------------------------------------------
 // One thread = 4 consecutive output pixels of a row x 32 channels (128 accumulators).  The weights are FFMA
 // constant-bank operands: with shared-memory weights the kernel ran at 36 % of its FP32 floor (two LDS.128 per
@@ -97,7 +97,7 @@ __global__ void pack_head_kernel(const float* __restrict__ w, float* __restrict_
 // host path; SURVEY.md N1).  The resize of image_pre_processing is the identity at the model's own resolution.
 template <bool U8>
 __global__ void __launch_bounds__(128) head_conv_kernel(const void* __restrict__ xin, int B, int D, int H, int W,
-                                                         __nv_bfloat16* __restrict__ out, int out_pitch) {
+                                                         __nv_bfloat16* __restrict__ out) {
   __shared__ float lut[U8 ? 256 : 1];
   if (U8) {
     for (int i = threadIdx.x; i < 256; i += blockDim.x)
@@ -171,13 +171,9 @@ __global__ void __launch_bounds__(128) head_conv_kernel(const void* __restrict__
       v1 = v1 > 0.f ? v1 : 0.01f * v1;
       op[i] = __floats2bfloat162_rn(v0, v1);
     }
-    uint4* dst = reinterpret_cast<uint4*>(out + (m0 + p) * out_pitch);
+    uint4* dst = reinterpret_cast<uint4*>(out + (m0 + p) * 32);
 #pragma unroll
     for (int i = 0; i < 4; ++i) dst[i] = o[i];
-    if (out_pitch == 64) {                       // zero-padded pitch: upper half zero
-#pragma unroll
-      for (int i = 4; i < 8; ++i) dst[i] = make_uint4(0u, 0u, 0u, 0u);
-    }
   }
 }
 
@@ -239,14 +235,13 @@ __global__ void __launch_bounds__(256) head_prep_kernel(const void* __restrict__
 // kernel skips (HaloArgs::tap_mask) -- 6 MMA instructions per input slice instead of 9 for the warp that issues them.
 // (Pairing kw = 1 with kw = 2, not kw = 0 with kw = 1: the row of tap kw = 0 of output column 0 lies left of the image and
 // is zero-filled as a whole by TMA, upper half included; the right neighbour of the last column is the stored zero pixel.)
-__global__ void head_split_weights_kernel(const float* __restrict__ w, float* __restrict__ out, int nine_taps) {
+__global__ void head_split_weights_kernel(const float* __restrict__ w, float* __restrict__ out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= 32 * 16 * 27) return;
   const int tap = i % 27, c16 = (i / 27) % 16, n = i / (27 * 16);
   const int kw = tap % 3, c = c16 & 7;
   int src_tap = -1;
-  if (nine_taps) src_tap = (c16 < 8) ? tap : -1;            // A/B switch V2CE_HEAD_9TAPS=1: every tap on its own, upper half zero
-  else if (c16 < 8) src_tap = (kw == 2) ? -1 : tap;         // kw = 0 and kw = 1 keep their own weights in the lower half
+  if (c16 < 8) src_tap = (kw == 2) ? -1 : tap;              // kw = 0 and kw = 1 keep their own weights in the lower half
   else src_tap = (kw == 1) ? tap + 1 : -1;                  // upper half of kw = 1: the weights of kw = 2 (next pixel)
   float v = 0.f;
   if (src_tap >= 0 && c < 6) {
@@ -397,28 +392,20 @@ __global__ void __launch_bounds__(256) sn_finish_kernel(const SnDesc* __restrict
 // ------------------------------------------------------------------------------------------
 // model
 // ------------------------------------------------------------------------------------------
-// Which kernel runs a layer and how its (virtual-concat) input channels are laid out in memory:
-// activations with fewer than 64 channels are stored with a 64-channel pitch (zeros above), so that
-// every TMA box row is a full 128-byte swizzle row; the packed weights carry zeros for the padding.
+// Which kernel runs a layer and how its (virtual-concat) input channels are laid out in memory.  Every activation
+// is stored densely: its channel pitch is its channel count.  32-channel tensors (64 B per pixel) are presented by
+// their TMA maps as 64-channel rows whose upper half is the NEXT pixel (conv_halo.cuh make_patch_map), which the
+// kernels never multiply (K=16 steps beyond the real channels are skipped); the packed weights carry zeros there.
 struct LayerCfg {
   int kind;                 // 0 direct fp32 (head, pred), 1 gather implicit GEMM (conv_igemm), 2 halo-tile (conv_halo)
   int pad0, real0, pad1, real1;   // channels per source in the packed K dimension (pad) and how many are real
-  int pitch0, pitch1;             // channel pitch of each source in memory
 };
 
 // K-chunk padding: the halo kernels multiply 64-channel chunks (one 128-byte swizzle row per pixel)
 static inline int chunk_of(int c) { return c < 64 ? 64 : c; }
-// Memory pitch of a c-channel activation.  32-channel tensors are stored densely (64 B per pixel); their TMA maps
-// present them as 64-channel rows whose upper half is the NEXT pixel (conv_halo.cuh make_patch_map), which the
-// kernels never multiply (K=16 steps beyond the real channels are skipped).  Halves the HBM traffic of the
-// full-resolution 32-channel tensors.  V2CE_PITCH64=1 restores the zero-padded 64-channel pitch.
-static inline int pitch_of(int c) {
-  static const bool p64 = getenv("V2CE_PITCH64") && atoi(getenv("V2CE_PITCH64"));
-  return (c < 64 && p64) ? 64 : c;
-}
 
 struct DevLayer {
-  LayerCfg cfg{0, 0, 0, 0, 0, 0, 0};
+  LayerCfg cfg{0, 0, 0, 0, 0};
   __nv_bfloat16* wpack = nullptr;
   __nv_bfloat16* wpack_kdm = nullptr;   // depth-merged packing (conv_halo_kdm.cuh) for halo layers with Cout <= 64
   float* scale = nullptr;
@@ -539,12 +526,12 @@ static Buffers carve(void* ws, const Dims& d) {
   Buffers b;
   static const int ch[5] = {32, 64, 128, 256, 512};
   b.head_in = a.take<__nv_bfloat16>(((size_t)d.M[0] + (size_t)d.M[0] / d.W[0] + 8) * 8 + 64);   // split-bf16 input pixels, rows of W+1 (last one zero)
-  b.head = a.take<__nv_bfloat16>((size_t)d.M[0] * pitch_of(32) + 64);  // 32 channels (+ the overlapped TMA view's reach)
+  b.head = a.take<__nv_bfloat16>((size_t)d.M[0] * 32 + 64);  // 32 channels (+ the overlapped TMA view's reach)
   for (int i = 0; i < 4; ++i) b.enc[i] = a.take<__nv_bfloat16>((size_t)d.M[i + 1] * ch[i + 1]);
   for (int i = 0; i < 2; ++i) b.res[i] = a.take<__nv_bfloat16>((size_t)d.M[4] * 512);
   for (int i = 0; i < 4; ++i) b.dec[i] = a.take<__nv_bfloat16>((size_t)d.M[3 - i] * ch[3 - i]);
   size_t tmax = 0, umax = 0;
-  for (int i = 0; i < 5; ++i) tmax = tmax > (size_t)d.M[i] * pitch_of(ch[i]) ? tmax : (size_t)d.M[i] * pitch_of(ch[i]);
+  for (int i = 0; i < 5; ++i) tmax = tmax > (size_t)d.M[i] * ch[i] ? tmax : (size_t)d.M[i] * ch[i];
   for (int i = 0; i < 4; ++i) umax = umax > (size_t)d.M[i] * ch[i + 1] ? umax : (size_t)d.M[i] * ch[i + 1];
   b.tmp_t = a.take<__nv_bfloat16>(tmax);
   b.tmp_r = a.take<__nv_bfloat16>(tmax);
@@ -564,11 +551,11 @@ static int layer_index(const char* name) {
 static LayerCfg layer_cfg(int li) {
   const LayerSpec& L = kLayers[li];
   const std::string n = L.name;
-  if (li == 0 || li == kNumLayers - 1) return LayerCfg{0, 0, 0, 0, 0, 0, 0};
+  if (li == 0 || li == kNumLayers - 1) return LayerCfg{0, 0, 0, 0, 0};
   const bool is_conv2 = n.find(".conv2") != std::string::npos;
   const bool is_dec = n.find("decoders") != std::string::npos;
   const bool is_enc = n.find("encoders") != std::string::npos;
-  LayerCfg c{1, 0, 0, 0, 0, 0, 0};
+  LayerCfg c{1, 0, 0, 0, 0};
   if (is_conv2) {
     c.kind = 2;
     c.real0 = L.cin;
@@ -580,8 +567,6 @@ static LayerCfg layer_cfg(int li) {
     c.kind = (L.k == 3 && !is_enc) ? 2 : 1;
     c.real0 = L.cin;
   }
-  c.pitch0 = pitch_of(c.real0);
-  c.pitch1 = c.real1 ? pitch_of(c.real1) : 0;
   // the halo kernel multiplies whole 64-channel TMA rows (padding channels carry zero weights and are skipped
   // at K=16 granularity); the gather kernel addresses real channels through the pitch
   c.pad0 = (c.kind == 2) ? chunk_of(c.real0) : c.real0;
@@ -624,9 +609,9 @@ static int run_conv(v2ce_model* m, int li, const __nv_bfloat16* src0, int c0, in
   a.inv_sigma = dl.sn_index >= 0 ? m->inv_sigma_dev + dl.sn_index : nullptr;
   a.residual = residual; a.out = out; a.act = act;
   a.error_flag = m->error_flag_dev;
-  if (dl.cfg.kind != 1 || c0 != dl.cfg.pitch0 || c1 != dl.cfg.pitch1)
+  if (dl.cfg.kind != 1 || c0 != dl.cfg.real0 || c1 != dl.cfg.real1)
     return set_error(V2CE_ERR_STATE, "layer %s: gather launch with pitches %d+%d, expected %d+%d", L.name, c0, c1,
-                     dl.cfg.pitch0, dl.cfg.pitch1);
+                     dl.cfg.real0, dl.cfg.real1);
   return conv::launch_conv(a, dl.bn_tile, s);
 }
 
@@ -637,14 +622,13 @@ static int run_halo(v2ce_model* m, int li, const __nv_bfloat16* src0, int p0, co
                     __nv_bfloat16* short_out = nullptr, int short_pitch = 0, bool* short_done = nullptr) {
   const LayerSpec& L = kLayers[li];
   const DevLayer& dl = m->layers[li];
-  if (dl.cfg.kind != 2 || p0 != dl.cfg.pitch0 || p1 != dl.cfg.pitch1)
+  if (dl.cfg.kind != 2 || p0 != dl.cfg.real0 || p1 != dl.cfg.real1)
     return set_error(V2CE_ERR_STATE, "layer %s: halo launch with pitches %d+%d, expected %d+%d", L.name, p0, p1,
-                     dl.cfg.pitch0, dl.cfg.pitch1);
+                     dl.cfg.real0, dl.cfg.real1);
   const halo::HaloPlan plan = halo::plan_for(dl.bn_tile, D, H, W);
   // layers with few output channels: depth taps merged into the MMA N dimension (conv_halo_kdm.cuh)
   const halo::KdmPlan kplan = halo::plan_kdm(D, H, W);
-  static const int kdm_max_cout = getenv("V2CE_KDM_MAX_COUT") ? atoi(getenv("V2CE_KDM_MAX_COUT")) : 64;
-  const bool kdm = dl.wpack_kdm != nullptr && kplan.ok && L.cout <= kdm_max_cout;
+  const bool kdm = dl.wpack_kdm != nullptr && kplan.ok;     // packed for Cout <= 64 (pack_layer)
   halo::HaloArgs a;
   a.a_row16 = 8; a.a_desc_hi = 0x40004040u;      // 64-channel SWIZZLE_128B patch rows
   a.tap_mask = 0x1FF;
@@ -681,8 +665,7 @@ static int run_halo(v2ce_model* m, int li, const __nv_bfloat16* src0, int p0, co
   if (short_done) *short_done = false;
   if (kdm) {
     // fuse the block's 1x1x1 shortcut conv (layer short_li) when asked for and packed
-    static const bool fuse = !(getenv("V2CE_NO_FUSED_SHORTCUT") && atoi(getenv("V2CE_NO_FUSED_SHORTCUT")));
-    if (short_li >= 0 && fuse && m->layers[short_li].wpack_kdm != nullptr) {
+    if (short_li >= 0 && m->layers[short_li].wpack_kdm != nullptr) {
       const DevLayer& sl = m->layers[short_li];
       halo::KdmShort sc{sl.wpack_kdm, sl.scale, sl.shift, short_out, short_pitch};
       if (short_done) *short_done = true;
@@ -702,10 +685,9 @@ static int run_enc_kdm(v2ce_model* m, int li, const __nv_bfloat16* x, int pin, i
   const DevLayer& dl = m->layers[li];
   const DevLayer& sl = m->layers[li + 2];
   *done = false;
-  static const bool off = getenv("V2CE_NO_S2_KDM") && atoi(getenv("V2CE_NO_S2_KDM"));
   const int Hout = (Hin - 1) / 2 + 1, Wout = (Win - 1) / 2 + 1;
   const halo::KdmPlan kp = halo::plan_kdm(D, Hout, Wout, 2);
-  if (off || !kp.ok || dl.wpack_kdm == nullptr || sl.wpack_kdm == nullptr || Hin < 2 || Win < 2) return V2CE_OK;
+  if (!kp.ok || dl.wpack_kdm == nullptr || sl.wpack_kdm == nullptr || Hin < 2 || Win < 2) return V2CE_OK;
   halo::HaloArgs a;
   a.a_row16 = 8; a.a_desc_hi = 0x40004040u;      // 64-channel SWIZZLE_128B patch rows
   a.tap_mask = 0x1FF;
@@ -747,16 +729,14 @@ static int pack_layer(v2ce_model* m, int li, const float* w_dev, cudaStream_t s)
   const int taps = L.k * L.k * L.k;
   const int cin_pad = c.pad0 + c.pad1;
   dl.bn_tile = conv::pick_bn(L.cout);
-  if (c.kind == 2 && dl.bn_tile == 256) {
+  if (c.kind == 2 && L.cout == 256) {
     // N tile of the 256- / 512-channel halo layers.  256-channel layers run as two N = 128 tiles: at 33 x 44 x 16 x 4
     // an N = 256 launch has 448 items = 3.03 waves of 148 CTAs (a quarter of the last wave's time is 4 items), the
     // N = 128 launch has 896 half-size items = 6.05 waves (3.5 full-item times) and a double-buffered accumulator, so
     // the epilogue overlaps the next item: encoders.2.conv2 0.326 -> 0.268 ms, decoders.0.conv1 0.823 -> 0.753,
     // decoders.0.conv2 0.381 -> 0.278 (profiles/layer_times_r2_l_*.txt).  512-channel layers (256 items = 1.73 waves
-    // either way) gain nothing and stay at 256.  V2CE_BN_COUT256 / V2CE_BN_COUT512 = 128 | 256 override.
-    const char* e = getenv(L.cout == 256 ? "V2CE_BN_COUT256" : "V2CE_BN_COUT512");
-    const int want = e ? atoi(e) : (L.cout == 256 ? 128 : 256);
-    if (want == 128) dl.bn_tile = 128;
+    // either way) gain nothing and stay at 256.
+    dl.bn_tile = 128;
   }
   if (c.real0 + c.real1 != L.cin) return set_error(V2CE_ERR_STATE, "layer %s: channel split mismatch", L.name);
   if (c.kind == 2) {
@@ -879,8 +859,7 @@ extern "C" int v2ce_model_finalize(v2ce_model* m) {
         // tensor-pipe variant: split weights in the depth-merged packing, unit scale, bias as shift
         float* w8 = nullptr;
         if (int e = dev_alloc(m, &w8, (size_t)32 * 16 * 27)) return e;
-        head_split_weights_kernel<<<(32 * 16 * 27 + 255) / 256, 256, 0, s>>>(
-            dl.w32, w8, (getenv("V2CE_HEAD_9TAPS") && atoi(getenv("V2CE_HEAD_9TAPS"))) ? 1 : 0);
+        head_split_weights_kernel<<<(32 * 16 * 27 + 255) / 256, 256, 0, s>>>(dl.w32, w8);
         V2CE_LAUNCH_CHECK("head_split_weights_kernel");
         if (int e = dev_alloc(m, &dl.wpack_kdm, (size_t)32 * 27 * 64)) return e;
         halo::pack_weights_kdm_kernel<<<(32 * 27 * 64 + 255) / 256, 256, 0, s>>>(w8, 32, 16, 64, 16, 0, 0, dl.wpack_kdm);
@@ -1006,10 +985,9 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
   launches += 4;
 
   const long long M0 = d.M[0];
-  static const bool head_direct = getenv("V2CE_HEAD_DIRECT") && atoi(getenv("V2CE_HEAD_DIRECT"));
   // 32-byte patch rows: 16-channel SWIZZLE_32B view of the 8-channel split pixels
   const halo::KdmPlan hplan = halo::plan_kdm(D, H, W, 1, 32);
-  if (hplan.ok && !head_direct) {
+  if (hplan.ok) {
     // head conv on the tensor pipe (see head_prep_kernel): split-bf16 pixels -> depth-merged halo kernel, LeakyReLU
     const size_t total = (size_t)M0;
     const int pgrid = (int)((total + 255) / 256 > 148 * 16 ? 148 * 16 : (total + 255) / 256);
@@ -1026,8 +1004,8 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     a.tiles_h = (H + a.TH - 1) / a.TH;
     a.ncc0 = 1; a.ncc1 = 0; a.real0 = 8; a.real1 = 0;
     // taps (kh, 0) and (kh, 1): the kw = 2 weights ride in the upper half of kw = 1
-    a.tap_mask = (getenv("V2CE_HEAD_9TAPS") && atoi(getenv("V2CE_HEAD_9TAPS"))) ? 0x1FF : 0x0DB;
-    a.Cout = 32; a.out_pitch = pitch_of(32); a.res_pitch = 0;
+    a.tap_mask = 0x0DB;
+    a.Cout = 32; a.out_pitch = 32; a.res_pitch = 0;
     a.T = halo::kKdmT; a.SA = hplan.SA; a.SB = 9; a.a_stage_bytes = hplan.a_stage_bytes; a.box_bytes = hplan.box_bytes;
     a.wpack = dl.wpack_kdm; a.scale = dl.scale; a.shift = dl.shift; a.inv_sigma = nullptr;
     a.residual = nullptr; a.out = buf.head; a.act = 2;
@@ -1058,9 +1036,9 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
       head_owner[m->device & 63] = m->uid;
     }
     if (frames_u8)
-      head_conv_kernel<true><<<(int)((groups + 127) / 128), 128, 0, s>>>(x_dev, B, D, H, W, buf.head, pitch_of(32));
+      head_conv_kernel<true><<<(int)((groups + 127) / 128), 128, 0, s>>>(x_dev, B, D, H, W, buf.head);
     else
-      head_conv_kernel<false><<<(int)((groups + 127) / 128), 128, 0, s>>>(x_dev, B, D, H, W, buf.head, pitch_of(32));
+      head_conv_kernel<false><<<(int)((groups + 127) / 128), 128, 0, s>>>(x_dev, B, D, H, W, buf.head);
     V2CE_LAUNCH_CHECK("head_conv_kernel");
   }
   ++launches;
@@ -1074,7 +1052,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
   for (int i = 0; i < 4; ++i) {
     snprintf(name, sizeof(name), "UNet.encoders.%d.conv1", i);
     const int l1 = layer_index(name);
-    const int pin = pitch_of(ch[i]), co = ch[i + 1];
+    const int pin = ch[i], co = ch[i + 1];
     bool fused = false;
     if (int e = run_enc_kdm(m, l1, x, pin, B, D, d.H[i], d.W[i], buf.tmp_t, buf.tmp_r, s, &fused)) return e;
     if (fused) {
@@ -1097,7 +1075,6 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
   }
   // residual blocks at the bottleneck (first spectral-norm convs: join the side stream here)
   V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_join, 0));
-  static const bool side_ok = !(getenv("V2CE_NO_SIDE_SHORTCUT") && atoi(getenv("V2CE_NO_SIDE_SHORTCUT")));
   int side_ev = 0;
   for (int i = 0; i < 2; ++i) {
     snprintf(name, sizeof(name), "UNet.resblocks.%d.conv1", i);
@@ -1105,7 +1082,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     // conv1 (persistent CTAs, a partial last wave) and the block's shortcut both read x: the shortcut goes to the
     // side stream AFTER conv1 so that its CTAs fill the SMs conv1 frees in its tail; conv2 waits for it.
     // (With per-launch timing on, everything stays on one stream.)
-    const bool side = !m->layer_timing && side_ok;
+    const bool side = !m->layer_timing;
     if (side) {
       V2CE_CUDA_CHECK(cudaEventRecord(m->ev_side[side_ev], s));
       V2CE_CUDA_CHECK(cudaStreamWaitEvent(m->sn_stream, m->ev_side[side_ev], 0));
@@ -1143,21 +1120,21 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
   for (int i = 0; i < 4; ++i) {
     const int lvl = 3 - i;                       // output level
     const __nv_bfloat16* skip = lvl == 0 ? buf.head : buf.enc[lvl - 1];
-    const int sp = pitch_of(ch[lvl]), co = ch[lvl], tp = pitch_of(co);
+    const int co = ch[lvl];                      // channels of the skip and of the outputs
     snprintf(name, sizeof(name), "UNet.decoders.%d.conv1", i);
     const int l1 = layer_index(name);
     bool short_done = false;
-    const bool side = !m->layer_timing && side_ok && side_ev + 2 <= 16;
+    const bool side = !m->layer_timing && side_ev + 2 <= 16;
     if (side) {
       V2CE_CUDA_CHECK(cudaEventRecord(m->ev_side[side_ev], s));
       V2CE_CUDA_CHECK(cudaStreamWaitEvent(m->sn_stream, m->ev_side[side_ev], 0));
     }
-    if (int e = run_halo(m, l1, up_cur, xc, skip, sp, B, D, d.H[lvl], d.W[lvl], nullptr, 0, 1, buf.tmp_t, tp, s, 0, 0, nullptr,
+    if (int e = run_halo(m, l1, up_cur, xc, skip, co, B, D, d.H[lvl], d.W[lvl], nullptr, 0, 1, buf.tmp_t, co, s, 0, 0, nullptr,
                          l1 + 2, buf.tmp_r, co, &short_done)) return e;
     mark(kLayers[l1].name);
     if (stop_at(l1, short_done ? l1 + 2 : -1)) return stop();
     if (!short_done) {
-      if (int e = run_conv(m, l1 + 2, up_cur, xc, d.H[lvl], d.W[lvl], skip, sp, B, D, d.H[lvl], d.W[lvl], 1, nullptr, 0, buf.tmp_r,
+      if (int e = run_conv(m, l1 + 2, up_cur, xc, d.H[lvl], d.W[lvl], skip, co, B, D, d.H[lvl], d.W[lvl], 1, nullptr, 0, buf.tmp_r,
                            side ? m->sn_stream : s)) return e;
       mark(kLayers[l1 + 2].name);
       ++launches;
@@ -1169,10 +1146,10 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     }
     if (side) side_ev += 2;
     if (lvl > 0) {
-      if (int e = run_halo(m, l1 + 1, buf.tmp_t, tp, nullptr, 0, B, D, d.H[lvl], d.W[lvl], buf.tmp_r, co, 1, up_next, co, s,
+      if (int e = run_halo(m, l1 + 1, buf.tmp_t, co, nullptr, 0, B, D, d.H[lvl], d.W[lvl], buf.tmp_r, co, 1, up_next, co, s,
                            d.H[lvl - 1], d.W[lvl - 1])) return e;
     } else {
-      if (int e = run_halo(m, l1 + 1, buf.tmp_t, tp, nullptr, 0, B, D, d.H[lvl], d.W[lvl], buf.tmp_r, co, 1, buf.dec[i], co, s,
+      if (int e = run_halo(m, l1 + 1, buf.tmp_t, co, nullptr, 0, B, D, d.H[lvl], d.W[lvl], buf.tmp_r, co, 1, buf.dec[i], co, s,
                            0, 0, y_dev)) return e;
     }
     mark(kLayers[l1 + 1].name);
