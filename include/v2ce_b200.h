@@ -152,8 +152,9 @@ int v2ce_baseline_emit(const float* voxels_dev, const v2ce_baseline_params* p, c
 /* ---- stage-2 evaluation metric (SURVEY.md 8f N4) ------------------------------------------------------------------
  * Replaces /root/reference/train/scripts/stage2/stage2_metrics.py:22-88 (ts_diff_metric): for every ground-truth event the
  * smallest |t_pred - t_gt| over the predicted events of the same polarity at the pixels within search_range (clamped to
- * the width x height sensor), capped at cap_us = 1e6/fps/10*3.  Both event sets are packed 13-byte records on the device
- * (ground-truth polarity -1 counts as 0, :38-41).  result_dev: int64[4] = {sum of the uncapped integer distances, number
+ * the width x height sensor; 0 <= search_range < 64), clamped to 1e6 (also when the window is empty) and capped at
+ * cap_us = 1e6/fps/10*3.  Both event sets are packed 13-byte records on the device (ground-truth polarity -1 counts as
+ * 0, :38-41).  result_dev: int64[4] = {sum of the clamped integer distances that are not capped, number
  * of capped ground-truth events ("overflow"), ground-truth events outside the sensor, predicted events outside the
  * sensor}; the metric is (result[0] + result[1] * cap_us) / n_gt. */
 int v2ce_ts_diff_workspace_bytes(int32_t width, int32_t height, int64_t n_pred, size_t* bytes);

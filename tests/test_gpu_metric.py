@@ -24,7 +24,9 @@ def _events(n, seed, spread, box=((90, 130), (40, 80)), neg_polarity=False):
     return ev
 
 
-@pytest.mark.parametrize('search_range,fps,n', [(0, 30, 2000), (1, 30, 2000), (3, 120, 1500), (0, 30, 1)])
+# fps 0.25 / 0.3: the cap is >= 1e6, so the 1 126 (r = 0) and 14 (r = 1) ground-truth events with an empty window add 1e6
+@pytest.mark.parametrize('search_range,fps,n', [(0, 30, 2000), (1, 30, 2000), (3, 120, 1500), (0, 30, 1), (0, 0.25, 2000),
+                                                (1, 0.3, 2000)])
 def test_metric_equals_oracle(search_range, fps, n):
     from v2ce_toolbox_b200.stage2_metrics import ts_diff_metric
     gt = _events(n, 1, 60000, neg_polarity=True)

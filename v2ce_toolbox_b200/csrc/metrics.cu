@@ -105,9 +105,10 @@ __global__ void ts_diff_kernel(const uint8_t* __restrict__ gt, long long n, int 
             best = ad < best ? ad : best;
           }
         }
-      // stage2_metrics.py:61,73-75: diff starts at 1e6 and is capped when it exceeds 1e6/fps/10*3
-      const double diff = (best == LLONG_MAX || (double)best > 1e6) ? 1e6 : (double)best;
-      if (diff > cap) over = 1ull; else sum = (unsigned long long)best;
+      // stage2_metrics.py:61,73-75: diff starts at 1e6 (no predicted event in the window, or none closer than 1e6 us)
+      // and is capped when it exceeds 1e6/fps/10*3; at fps <= 0.3 the cap is >= 1e6, so the clamped value is what adds up
+      const long long d = best > 1000000 ? 1000000 : best;
+      if ((double)d > cap) over = 1ull; else sum = (unsigned long long)d;
     }
   }
   // block reduction, three atomics per block
