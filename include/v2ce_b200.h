@@ -234,29 +234,22 @@ int v2ce_model_last_launches(const v2ce_model* m, int32_t* launches);
 /* Layer-level hook used by the parity tests: one fused conv launch.
  *  src0 (B,D,H0,W0,C0) bf16 [nearest-upsampled to (Hin,Win) when H0!=Hin], src1 (B,D,Hin,Win,C1) bf16 or NULL,
  *  weight_host (Cout, C0+C1, k,k,k) float32, scale/shift float32[Cout] (host), residual (M,Cout) bf16 or NULL,
- *  act: 0 none, 1 relu, 2 leaky_relu(0.01).  out (B,D,Hout,Wout,Cout) bf16. */
-int v2ce_conv3d_bf16(const void* src0_dev, int32_t c0, int32_t h0, int32_t w0, const void* src1_dev, int32_t c1,
-                     int32_t batch, int32_t depth, int32_t hin, int32_t win, int32_t ksize, int32_t stride_hw,
-                     const float* weight_host, int32_t cout, const float* scale_host, const float* shift_host,
-                     const void* residual_dev, int32_t act, void* out_dev, void* stream);
-
-/* Same hook with the kernel made explicit: impl 0 = gather implicit GEMM (csrc/conv_igemm.cuh), 1 = halo-tile
- * kernel (csrc/conv_halo.cuh; 3x3x3, stride 1, h0==hin, channel pitches multiple of 64), 2 = its depth-merged
- * variant (csrc/conv_halo_kdm.cuh; additionally Cout <= 64, depth % 8 == 0), 3 = the same with the fused 1x1x1
- * shortcut: residual_dev is then an OUTPUT (B,D,H,W,Cout) bf16 receiving scale*conv1x1(x, weight[:,:,1,1,1])+shift.
- * desc_mode is a bring-up switch of the shifted shared-memory descriptor (0 or 1). */
+ *  act: 0 none, 1 relu, 2 leaky_relu(0.01).  out (B,D,Hout,Wout,Cout) bf16.
+ *  impl selects the kernel: 0 = gather implicit GEMM (csrc/conv_igemm.cuh), 1 = halo-tile kernel
+ *  (csrc/conv_halo.cuh; 3x3x3, stride 1, h0==hin, channel pitches multiple of 64), 2 = its depth-merged variant
+ *  (csrc/conv_halo_kdm.cuh; additionally Cout <= 64, depth % 8 == 0), 3 = the same with the fused 1x1x1 shortcut:
+ *  residual_dev is then an OUTPUT (B,D,H,W,Cout) bf16 receiving scale*conv1x1(x, weight[:,:,1,1,1])+shift. */
 int v2ce_conv3d_bf16_ex(const void* src0_dev, int32_t c0, int32_t h0, int32_t w0, const void* src1_dev, int32_t c1,
                         int32_t batch, int32_t depth, int32_t hin, int32_t win, int32_t ksize, int32_t stride_hw,
                         const float* weight_host, int32_t cout, const float* scale_host, const float* shift_host,
-                        const void* residual_dev, int32_t act, void* out_dev, int32_t impl, int32_t desc_mode,
-                        void* stream);
+                        const void* residual_dev, int32_t act, void* out_dev, int32_t impl, void* stream);
 /* Bring-up microbenchmark: cycles per back-to-back tcgen05.mma (M=128, N=bn, K=16, both operands in shared
  * memory) with `naccs` accumulators in rotation on `ctas` CTAs. */
 int v2ce_debug_mma_rate(int32_t bn, int32_t iters, int32_t naccs, int32_t ctas, double* cycles_per_mma);
 /* Per-launch device times of the last forward, measured with CUDA events on the launch stream when the option
  * "layer_timing" is 1: ms_out[i] and the layer name (48 bytes each, NUL terminated) of launch i. */
 int v2ce_model_layer_times(v2ce_model* m, int32_t cap, float* ms_out, char* names_out, int32_t* count);
-/* Tuning / bring-up options of a model handle: "desc_mode", "layer_timing", and "stop_after" (per-layer tests; default
+/* Tuning / bring-up options of a model handle: "layer_timing", and "stop_after" (per-layer tests; default
  * -1 = off): a layer index in state-dict order (head 0 .. pred 31); the forward returns right after the launch that
  * writes that layer's output, with every stream it used joined into `stream`.  A block's shortcut fused into its conv1
  * stops after that launch, pred after decoders.3.conv2.  The workspace then holds the layer's inputs and its output. */

@@ -14,7 +14,7 @@ from conftest import record_measurement
 pytestmark = pytest.mark.gpu
 
 
-def conv_hook(src0, src1, hin, win, w, scale, shift, residual, act, ksize, stride, impl=0, desc_mode=0):
+def conv_hook(src0, src1, hin, win, w, scale, shift, residual, act, ksize, stride, impl=0):
     """src0 (B,D,H0,W0,C0) bf16, src1 (B,D,Hin,Win,C1) bf16 | None -> out (B,D,Hout,Wout,Cout) bf16."""
     from v2ce_toolbox_b200 import _lib
     lib = _lib.load()
@@ -31,7 +31,7 @@ def conv_hook(src0, src1, hin, win, w, scale, shift, residual, act, ksize, strid
     _lib.check(lib.v2ce_conv3d_bf16_ex(_lib.ptr(src0), C0, H0, W0, _lib.ptr(src1), C1, B, D, hin, win, ksize, stride,
                                        wh.ctypes.data_as(ctypes.c_void_p), cout, sh.ctypes.data_as(ctypes.c_void_p),
                                        th.ctypes.data_as(ctypes.c_void_p), _lib.ptr(residual), act, _lib.ptr(out),
-                                       impl, desc_mode, _lib.stream_ptr()))
+                                       impl, _lib.stream_ptr()))
     torch.cuda.synchronize()
     return out
 

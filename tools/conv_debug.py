@@ -8,7 +8,7 @@ import torch
 import test_gpu_unet as T
 
 
-def main(name, impl=0, desc_mode=0):
+def main(name, impl=0):
     case = [c for c in T.CASES + T.HALO_CASES + T.KDM_CASES if c[0] == name][0]
     _, B, D, hin, win, C0, up, C1, cout, k, stride, use_res, act = case
     g = torch.Generator(device='cpu').manual_seed(hash(name) % 1000)
@@ -23,7 +23,7 @@ def main(name, impl=0, desc_mode=0):
     hout, wout = (hin + 2 * pad - k) // stride + 1, (win + 2 * pad - k) // stride + 1
     res = torch.randn(B, D, hout, wout, cout, generator=g).to(torch.bfloat16).cuda() if use_res else None
     try:
-        out = T.conv_hook(src0, src1, hin, win, w, scale, shift, res, act, k, stride, impl=impl, desc_mode=desc_mode)
+        out = T.conv_hook(src0, src1, hin, win, w, scale, shift, res, act, k, stride, impl=impl)
     except Exception as e:
         print(f'CASE {name}: EXCEPTION {e}')
         return 2
@@ -35,7 +35,7 @@ def main(name, impl=0, desc_mode=0):
     err[torch.isnan(err)] = 1e9
     tol = 2.0 ** -8 * r.abs() + 2e-3
     bad = err > tol
-    print(f'CASE {name} impl={impl} mode={desc_mode}: M={o.shape[0]} N={cout} K={cin * k ** 3} nan={nan} bad={bad.sum().item()}/{bad.numel()} '
+    print(f'CASE {name} impl={impl}: M={o.shape[0]} N={cout} K={cin * k ** 3} nan={nan} bad={bad.sum().item()}/{bad.numel()} '
           f'maxerr={err[~torch.isnan(o)].max().item() if nan < o.numel() else -1:.4g} refmax={r.abs().max().item():.3g}')
     if bad.any():
         rows = bad.any(dim=1).nonzero().flatten()
@@ -50,4 +50,4 @@ def main(name, impl=0, desc_mode=0):
 
 
 if __name__ == '__main__':
-    sys.exit(main(sys.argv[1], int(sys.argv[2]) if len(sys.argv) > 2 else 0, int(sys.argv[3]) if len(sys.argv) > 3 else 0))
+    sys.exit(main(sys.argv[1], int(sys.argv[2]) if len(sys.argv) > 2 else 0))

@@ -88,12 +88,9 @@ _SIGNATURES = {
     'v2ce_model_call_count': (c_int, [c_void_p, POINTER(c_int64)]),
     'v2ce_model_sn_advance': (c_int, [c_void_p, c_int32, c_void_p]),
     'v2ce_model_last_launches': (c_int, [c_void_p, POINTER(c_int32)]),
-    'v2ce_conv3d_bf16': (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32, c_int32, c_int32,
-                                 c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
-                                 c_int32, c_void_p, c_void_p]),
     'v2ce_conv3d_bf16_ex': (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32, c_int32, c_int32,
                                     c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
-                                    c_int32, c_void_p, c_int32, c_int32, c_void_p]),
+                                    c_int32, c_void_p, c_int32, c_void_p]),
     'v2ce_model_set_option': (c_int, [c_void_p, c_char_p, c_int64]),
     'v2ce_model_layer_times': (c_int, [c_void_p, c_int32, POINTER(c_float), c_char_p, POINTER(c_int32)]),
     'v2ce_debug_mma_rate': (c_int, [c_int32, c_int32, c_int32, c_int32, POINTER(c_double)]),

@@ -32,46 +32,52 @@ using conv::ConvArgs;
 constexpr float kBnEps = 1e-5f;
 constexpr int kNumSn = 12;
 
+// What a layer is in the network.  Its role decides its kernel, its channel split and its weight packings (layer_cfg,
+// pack_layer) and where forward_impl runs it.  A block's layers follow each other: conv1, conv2, shortcut.
+enum class Role { Head, EncConv1, EncShort, ResConv1, ResShort, DecConv1, DecShort, Conv2, Pred };
+
 struct LayerSpec {
   const char* name;
+  Role role;
+  int block;        // index of the encoder / resblock / decoder the layer belongs to
   int cin, cout, k;
   bool sn, bias;
   const char* bn;   // BatchNorm prefix or nullptr
 };
 
 static const LayerSpec kLayers[] = {
-    {"UNet.head.conv3d", 2, 32, 3, false, true, nullptr},
-    {"UNet.encoders.0.conv1", 32, 64, 3, false, false, "UNet.encoders.0.bn1"},
-    {"UNet.encoders.0.conv2", 64, 64, 3, false, false, "UNet.encoders.0.bn2"},
-    {"UNet.encoders.0.downsample.0", 32, 64, 1, false, true, "UNet.encoders.0.downsample.1"},
-    {"UNet.encoders.1.conv1", 64, 128, 3, false, false, "UNet.encoders.1.bn1"},
-    {"UNet.encoders.1.conv2", 128, 128, 3, false, false, "UNet.encoders.1.bn2"},
-    {"UNet.encoders.1.downsample.0", 64, 128, 1, false, true, "UNet.encoders.1.downsample.1"},
-    {"UNet.encoders.2.conv1", 128, 256, 3, false, false, "UNet.encoders.2.bn1"},
-    {"UNet.encoders.2.conv2", 256, 256, 3, false, false, "UNet.encoders.2.bn2"},
-    {"UNet.encoders.2.downsample.0", 128, 256, 1, false, true, "UNet.encoders.2.downsample.1"},
-    {"UNet.encoders.3.conv1", 256, 512, 3, false, false, "UNet.encoders.3.bn1"},
-    {"UNet.encoders.3.conv2", 512, 512, 3, false, false, "UNet.encoders.3.bn2"},
-    {"UNet.encoders.3.downsample.0", 256, 512, 1, false, true, "UNet.encoders.3.downsample.1"},
-    {"UNet.resblocks.0.conv1", 512, 512, 3, true, false, "UNet.resblocks.0.bn1"},
-    {"UNet.resblocks.0.conv2", 512, 512, 3, true, false, "UNet.resblocks.0.bn2"},
-    {"UNet.resblocks.0.downsample.0", 512, 512, 1, false, true, "UNet.resblocks.0.downsample.1"},
-    {"UNet.resblocks.1.conv1", 512, 512, 3, true, false, "UNet.resblocks.1.bn1"},
-    {"UNet.resblocks.1.conv2", 512, 512, 3, true, false, "UNet.resblocks.1.bn2"},
-    {"UNet.resblocks.1.downsample.0", 512, 512, 1, false, true, "UNet.resblocks.1.downsample.1"},
-    {"UNet.decoders.0.conv1", 768, 256, 3, true, false, "UNet.decoders.0.bn1"},
-    {"UNet.decoders.0.conv2", 256, 256, 3, true, false, "UNet.decoders.0.bn2"},
-    {"UNet.decoders.0.downsample.0", 768, 256, 1, false, true, "UNet.decoders.0.downsample.1"},
-    {"UNet.decoders.1.conv1", 384, 128, 3, true, false, "UNet.decoders.1.bn1"},
-    {"UNet.decoders.1.conv2", 128, 128, 3, true, false, "UNet.decoders.1.bn2"},
-    {"UNet.decoders.1.downsample.0", 384, 128, 1, false, true, "UNet.decoders.1.downsample.1"},
-    {"UNet.decoders.2.conv1", 192, 64, 3, true, false, "UNet.decoders.2.bn1"},
-    {"UNet.decoders.2.conv2", 64, 64, 3, true, false, "UNet.decoders.2.bn2"},
-    {"UNet.decoders.2.downsample.0", 192, 64, 1, false, true, "UNet.decoders.2.downsample.1"},
-    {"UNet.decoders.3.conv1", 96, 32, 3, true, false, "UNet.decoders.3.bn1"},
-    {"UNet.decoders.3.conv2", 32, 32, 3, true, false, "UNet.decoders.3.bn2"},
-    {"UNet.decoders.3.downsample.0", 96, 32, 1, false, true, "UNet.decoders.3.downsample.1"},
-    {"UNet.pred.conv3d", 32, 20, 1, false, true, nullptr},
+    {"UNet.head.conv3d", Role::Head, 0, 2, 32, 3, false, true, nullptr},
+    {"UNet.encoders.0.conv1", Role::EncConv1, 0, 32, 64, 3, false, false, "UNet.encoders.0.bn1"},
+    {"UNet.encoders.0.conv2", Role::Conv2, 0, 64, 64, 3, false, false, "UNet.encoders.0.bn2"},
+    {"UNet.encoders.0.downsample.0", Role::EncShort, 0, 32, 64, 1, false, true, "UNet.encoders.0.downsample.1"},
+    {"UNet.encoders.1.conv1", Role::EncConv1, 1, 64, 128, 3, false, false, "UNet.encoders.1.bn1"},
+    {"UNet.encoders.1.conv2", Role::Conv2, 1, 128, 128, 3, false, false, "UNet.encoders.1.bn2"},
+    {"UNet.encoders.1.downsample.0", Role::EncShort, 1, 64, 128, 1, false, true, "UNet.encoders.1.downsample.1"},
+    {"UNet.encoders.2.conv1", Role::EncConv1, 2, 128, 256, 3, false, false, "UNet.encoders.2.bn1"},
+    {"UNet.encoders.2.conv2", Role::Conv2, 2, 256, 256, 3, false, false, "UNet.encoders.2.bn2"},
+    {"UNet.encoders.2.downsample.0", Role::EncShort, 2, 128, 256, 1, false, true, "UNet.encoders.2.downsample.1"},
+    {"UNet.encoders.3.conv1", Role::EncConv1, 3, 256, 512, 3, false, false, "UNet.encoders.3.bn1"},
+    {"UNet.encoders.3.conv2", Role::Conv2, 3, 512, 512, 3, false, false, "UNet.encoders.3.bn2"},
+    {"UNet.encoders.3.downsample.0", Role::EncShort, 3, 256, 512, 1, false, true, "UNet.encoders.3.downsample.1"},
+    {"UNet.resblocks.0.conv1", Role::ResConv1, 0, 512, 512, 3, true, false, "UNet.resblocks.0.bn1"},
+    {"UNet.resblocks.0.conv2", Role::Conv2, 0, 512, 512, 3, true, false, "UNet.resblocks.0.bn2"},
+    {"UNet.resblocks.0.downsample.0", Role::ResShort, 0, 512, 512, 1, false, true, "UNet.resblocks.0.downsample.1"},
+    {"UNet.resblocks.1.conv1", Role::ResConv1, 1, 512, 512, 3, true, false, "UNet.resblocks.1.bn1"},
+    {"UNet.resblocks.1.conv2", Role::Conv2, 1, 512, 512, 3, true, false, "UNet.resblocks.1.bn2"},
+    {"UNet.resblocks.1.downsample.0", Role::ResShort, 1, 512, 512, 1, false, true, "UNet.resblocks.1.downsample.1"},
+    {"UNet.decoders.0.conv1", Role::DecConv1, 0, 768, 256, 3, true, false, "UNet.decoders.0.bn1"},
+    {"UNet.decoders.0.conv2", Role::Conv2, 0, 256, 256, 3, true, false, "UNet.decoders.0.bn2"},
+    {"UNet.decoders.0.downsample.0", Role::DecShort, 0, 768, 256, 1, false, true, "UNet.decoders.0.downsample.1"},
+    {"UNet.decoders.1.conv1", Role::DecConv1, 1, 384, 128, 3, true, false, "UNet.decoders.1.bn1"},
+    {"UNet.decoders.1.conv2", Role::Conv2, 1, 128, 128, 3, true, false, "UNet.decoders.1.bn2"},
+    {"UNet.decoders.1.downsample.0", Role::DecShort, 1, 384, 128, 1, false, true, "UNet.decoders.1.downsample.1"},
+    {"UNet.decoders.2.conv1", Role::DecConv1, 2, 192, 64, 3, true, false, "UNet.decoders.2.bn1"},
+    {"UNet.decoders.2.conv2", Role::Conv2, 2, 64, 64, 3, true, false, "UNet.decoders.2.bn2"},
+    {"UNet.decoders.2.downsample.0", Role::DecShort, 2, 192, 64, 1, false, true, "UNet.decoders.2.downsample.1"},
+    {"UNet.decoders.3.conv1", Role::DecConv1, 3, 96, 32, 3, true, false, "UNet.decoders.3.bn1"},
+    {"UNet.decoders.3.conv2", Role::Conv2, 3, 32, 32, 3, true, false, "UNet.decoders.3.bn2"},
+    {"UNet.decoders.3.downsample.0", Role::DecShort, 3, 96, 32, 1, false, true, "UNet.decoders.3.downsample.1"},
+    {"UNet.pred.conv3d", Role::Pred, 0, 32, 20, 1, false, true, nullptr},
 };
 constexpr int kNumLayers = sizeof(kLayers) / sizeof(kLayers[0]);
 
@@ -396,8 +402,14 @@ __global__ void __launch_bounds__(256) sn_finish_kernel(const SnDesc* __restrict
 // is stored densely: its channel pitch is its channel count.  32-channel tensors (64 B per pixel) are presented by
 // their TMA maps as 64-channel rows whose upper half is the NEXT pixel (conv_halo.cuh make_patch_map), which the
 // kernels never multiply (K=16 steps beyond the real channels are skipped); the packed weights carry zeros there.
+enum class Kernel {
+  Direct,                   // fp32 on CUDA cores (head, pred)
+  Gather,                   // gather implicit GEMM (conv_igemm.cuh)
+  Halo,                     // halo tiles (conv_halo.cuh, or conv_halo_kdm.cuh when packed for it)
+};
+
 struct LayerCfg {
-  int kind;                 // 0 direct fp32 (head, pred), 1 gather implicit GEMM (conv_igemm), 2 halo-tile (conv_halo)
+  Kernel kernel;
   int pad0, real0, pad1, real1;   // channels per source in the packed K dimension (pad) and how many are real
 };
 
@@ -405,14 +417,32 @@ struct LayerCfg {
 static inline int chunk_of(int c) { return c < 64 ? 64 : c; }
 
 struct DevLayer {
-  LayerCfg cfg{0, 0, 0, 0, 0};
+  LayerCfg cfg{Kernel::Direct, 0, 0, 0, 0};
   __nv_bfloat16* wpack = nullptr;
   __nv_bfloat16* wpack_kdm = nullptr;   // depth-merged packing (conv_halo_kdm.cuh) for halo layers with Cout <= 64
   float* scale = nullptr;
   float* shift = nullptr;
+  const float* inv_sigma = nullptr;     // spectral-norm layers: 1 / sigma on the device
   float* w32 = nullptr;     // head / pred fp32 weights, SN weight_bar
   float* bias = nullptr;    // head / pred bias
-  int bn_tile = 0, num_kb = 0, sn_index = -1;
+  int bn_tile = 0, num_kb = 0;
+};
+
+// The TMA views a halo launch reads its sources through: 64-channel patch rows (halo::make_patch_map), the head's
+// split pixels as 16-channel rows (make_patch_map16) or one of the four parity views of a stride-2 input
+// (make_parity_map).
+enum class View { Patch64, Head16, Parity };
+
+struct MapKey {
+  View view;
+  int q;                    // Parity: row parity * 2 + column parity
+  const void* ptr;
+  int B, D, H, W, cpitch;   // the tensor (B, D, H, W, cpitch)
+  int PW, rows;             // the box: PW pixels by `rows` rows
+  bool operator<(const MapKey& o) const {
+    return std::tie(view, q, ptr, B, D, H, W, cpitch, PW, rows) <
+           std::tie(o.view, o.q, o.ptr, o.B, o.D, o.H, o.W, o.cpitch, o.PW, o.rows);
+  }
 };
 
 }  // namespace unet
@@ -435,14 +465,13 @@ struct v2ce_model {
   int max_rows = 0, max_k = 0;
   int64_t calls = 0;
   int last_launches = 0;
-  int desc_mode = 0;
   int layer_timing = 0;                 // option "layer_timing": CUDA events around every launch of forward()
   int stop_after = -1;                  // option "stop_after" (per-layer tests): kLayers index, -1 = run the whole forward
   std::vector<std::pair<std::string, cudaEvent_t>> marks;
   cudaStream_t sn_stream = nullptr;     // the spectral-norm step overlaps the head / encoder convs
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   cudaEvent_t ev_side[16] = {nullptr};  // x-ready / shortcut-done pairs of the blocks whose shortcut runs on the side stream
-  std::map<std::tuple<const void*, int, int, int, int, int, int, int>, CUtensorMap> tmaps;
+  std::map<v2ce::unet::MapKey, CUtensorMap> tmaps;
 };
 
 namespace v2ce {
@@ -488,6 +517,7 @@ static bool known_name(const std::string& name) {
   return false;
 }
 
+constexpr int kSnLaunches = 4;   // kernels of one run_sn_step
 static int run_sn_step(v2ce_model* m, cudaStream_t s) {
   dim3 g1((m->max_k + kSnCols - 1) / kSnCols, kNumSn);
   sn_wtu_kernel<<<g1, 256, 0, s>>>(m->sn_descs_dev);
@@ -541,51 +571,119 @@ static Buffers carve(void* ws, const Dims& d) {
   return b;
 }
 
-static int layer_index(const char* name) {
+// kLayers index of the conv1 of block `block` with role r; the block's conv2 and shortcut follow it
+static int conv1_of(Role r, int block) {
   for (int i = 0; i < kNumLayers; ++i)
-    if (std::string(kLayers[i].name) == name) return i;
+    if (kLayers[i].role == r && kLayers[i].block == block) return i;
   return -1;
 }
 
 // kernel choice and channel padding per layer (see LayerCfg)
-static LayerCfg layer_cfg(int li) {
-  const LayerSpec& L = kLayers[li];
-  const std::string n = L.name;
-  if (li == 0 || li == kNumLayers - 1) return LayerCfg{0, 0, 0, 0, 0};
-  const bool is_conv2 = n.find(".conv2") != std::string::npos;
-  const bool is_dec = n.find("decoders") != std::string::npos;
-  const bool is_enc = n.find("encoders") != std::string::npos;
-  LayerCfg c{1, 0, 0, 0, 0};
-  if (is_conv2) {
-    c.kind = 2;
-    c.real0 = L.cin;
-  } else if (is_dec) {                       // conv1 / shortcut of a decoder: [up (2/3 of Cin) | skip (1/3)]
-    c.kind = (L.k == 3) ? 2 : 1;
-    c.real0 = L.cin / 3 * 2;
-    c.real1 = L.cin / 3;
-  } else {                                   // conv1 / shortcut of an encoder (stride 2) or bottleneck block
-    c.kind = (L.k == 3 && !is_enc) ? 2 : 1;
-    c.real0 = L.cin;
-  }
+static LayerCfg layer_cfg(const LayerSpec& L) {
+  if (L.role == Role::Head || L.role == Role::Pred) return LayerCfg{Kernel::Direct, 0, 0, 0, 0};
+  // encoder conv1 (stride 2) and the shortcuts run on the gather kernel
+  const bool halo = L.role == Role::Conv2 || L.role == Role::ResConv1 || L.role == Role::DecConv1;
+  // conv1 / shortcut of a decoder read [up (2/3 of Cin) | skip (1/3)]
+  const bool split = L.role == Role::DecConv1 || L.role == Role::DecShort;
+  LayerCfg c{halo ? Kernel::Halo : Kernel::Gather, 0, split ? L.cin / 3 * 2 : L.cin, 0, split ? L.cin / 3 : 0};
   // the halo kernel multiplies whole 64-channel TMA rows (padding channels carry zero weights and are skipped
   // at K=16 granularity); the gather kernel addresses real channels through the pitch
-  c.pad0 = (c.kind == 2) ? chunk_of(c.real0) : c.real0;
-  c.pad1 = (c.kind == 2) ? (c.real1 ? chunk_of(c.real1) : 0) : c.real1;
+  c.pad0 = halo ? chunk_of(c.real0) : c.real0;
+  c.pad1 = halo && c.real1 ? chunk_of(c.real1) : c.real1;
   return c;
 }
 
-static int get_tmap(v2ce_model* m, const void* ptr, int B, int D, int H, int W, int cpitch, int PW, int rows,
-                    CUtensorMap* out) {
-  auto key = std::make_tuple(ptr, B, D, H, W, cpitch, PW, rows);
+static int make_map(const MapKey& k, CUtensorMap* tm) {
+  switch (k.view) {
+    case View::Patch64: return halo::make_patch_map(tm, k.ptr, k.B, k.D, k.H, k.W, k.cpitch, k.PW, k.rows);
+    case View::Head16: return halo::make_patch_map16(tm, k.ptr, k.B, k.D, k.H, k.W, k.PW, k.rows);
+    case View::Parity:
+      return halo::make_parity_map(tm, k.ptr, k.B, k.D, k.H, k.W, k.cpitch, k.q >> 1, k.q & 1, k.PW, k.rows);
+  }
+  return set_error(V2CE_ERR_STATE, "unknown tensor-map view %d", (int)k.view);
+}
+
+// make_map, cached per handle.  The map is returned by value: clearing the cache invalidates nothing a caller holds.
+static int get_tmap(v2ce_model* m, const MapKey& key, CUtensorMap* out) {
   auto it = m->tmaps.find(key);
   if (it == m->tmaps.end()) {
     if (m->tmaps.size() > 512) m->tmaps.clear();      // callers that move their workspace every call must not grow the cache
     CUtensorMap tm;
-    if (int e = halo::make_patch_map(&tm, ptr, B, D, H, W, cpitch, PW, rows)) return e;
+    if (int e = make_map(key, &tm)) return e;
     it = m->tmaps.emplace(key, tm).first;
   }
   *out = it->second;
   return V2CE_OK;
+}
+
+// __constant__ memory is per device, not per handle: `load` (stream ordered) runs when another handle loaded this
+// image on the device last
+template <typename Load>
+static int load_constants(unsigned long long (&owner)[64], const v2ce_model* m, Load load) {
+  unsigned long long& o = owner[m->device & 63];
+  if (o == m->uid) return V2CE_OK;
+  if (int e = load()) return e;
+  o = m->uid;
+  return V2CE_OK;
+}
+
+// The one place that fills conv::ConvArgs: a gather implicit-GEMM launch (stride-2 convs, 1x1x1 shortcuts) of the
+// k x k x k layer `dl` with cout outputs; p0 / p1 are the channel PITCHES of the sources
+static ConvArgs conv_args(const DevLayer& dl, int k, int cout, const __nv_bfloat16* src0, int p0, int h0, int w0,
+                          const __nv_bfloat16* src1, int p1, int B, int D, int hin, int win, int stride,
+                          const __nv_bfloat16* residual, int act, __nv_bfloat16* out, int* error_flag) {
+  ConvArgs a;
+  a.src0 = src0; a.src1 = src1; a.C0 = dl.cfg.real0; a.C1 = dl.cfg.real1; a.Cin = a.C0 + a.C1;
+  a.P0 = p0; a.P1 = p1;
+  a.H0 = h0; a.W0 = w0; a.B = B; a.D = D; a.Hin = hin; a.Win = win;
+  a.stride = stride; a.ksize = k; a.pad = k / 2;
+  a.Hout = (hin + 2 * a.pad - k) / stride + 1;
+  a.Wout = (win + 2 * a.pad - k) / stride + 1;
+  a.taps = k * k * k;
+  a.num_kb = dl.num_kb;
+  a.M = B * D * a.Hout * a.Wout;
+  a.Cout = cout;
+  a.wpack = dl.wpack; a.scale = dl.scale; a.shift = dl.shift; a.inv_sigma = dl.inv_sigma;
+  a.residual = residual; a.out = out; a.act = act;
+  a.error_flag = error_flag;
+  return a;
+}
+
+// The one place that fills halo::HaloArgs: a launch of layer `dl` over the output plane (B, D, H, W) with cout outputs,
+// reading its sources through `view`.  With the depth-merged plan `kp` it runs conv_halo_kdm.cuh, otherwise
+// conv_halo.cuh with the plan `hp`.  The Head16 view carries the head's 8-channel split pixels (head_prep_kernel).
+static halo::HaloArgs halo_args(const DevLayer& dl, View view, const halo::HaloPlan* hp, const halo::KdmPlan* kp, int B,
+                                int D, int H, int W, int cout, __nv_bfloat16* out, int out_pitch,
+                                const __nv_bfloat16* residual, int res_pitch, int act, int* error_flag, int up_H = 0,
+                                int up_W = 0, const DevLayer* pred = nullptr, float* pred_out = nullptr) {
+  const bool head = view == View::Head16;
+  const halo::TileShape ts = kp ? kp->ts : hp->ts;
+  halo::HaloArgs a;
+  // 64-channel SWIZZLE_128B patch rows, or the head's K-major SWIZZLE_32B rows (8-row groups 256 B apart) with the
+  // taps (kh, 0) and (kh, 1) only: the kw = 2 weights ride in the upper half of kw = 1 (head_split_weights_kernel)
+  a.a_row16 = head ? 2 : 8;
+  a.a_desc_hi = head ? 0xC0004010u : 0x40004040u;
+  a.tap_mask = head ? 0x0DB : 0x1FF;
+  a.B = B; a.D = D; a.H = H; a.W = W;
+  a.PW = ts.PW; a.TH = ts.TH; a.TW = kp ? kp->TW : ts.PW - 2;
+  a.tiles_w = (W + a.TW - 1) / a.TW;
+  a.tiles_h = (H + a.TH - 1) / a.TH;
+  a.real0 = head ? 8 : dl.cfg.real0; a.real1 = dl.cfg.real1;
+  a.ncc0 = chunk_of(a.real0) / 64; a.ncc1 = a.real1 ? chunk_of(a.real1) / 64 : 0;
+  a.Cout = cout; a.out_pitch = out_pitch; a.res_pitch = res_pitch;
+  a.T = kp ? halo::kKdmT : hp->T;
+  a.SA = kp ? kp->SA : hp->SA;
+  a.SB = kp ? 9 : hp->SB;
+  a.a_stage_bytes = kp ? kp->a_stage_bytes : hp->a_stage_bytes;
+  a.box_bytes = kp ? kp->box_bytes : hp->box_bytes;
+  a.wpack = kp ? dl.wpack_kdm : dl.wpack; a.scale = dl.scale; a.shift = dl.shift; a.inv_sigma = dl.inv_sigma;
+  a.residual = residual; a.out = out; a.act = act;
+  a.up_H = up_H; a.up_W = up_W;
+  a.pred_w = pred ? pred->w32 : nullptr;
+  a.pred_b = pred ? pred->bias : nullptr;
+  a.pred_out = pred_out;
+  a.error_flag = error_flag;
+  return a;
 }
 
 // gather implicit-GEMM launch of layer `li` (stride-2 convs, 1x1x1 shortcuts); c0/c1 are channel PITCHES
@@ -594,25 +692,12 @@ static int run_conv(v2ce_model* m, int li, const __nv_bfloat16* src0, int c0, in
                     __nv_bfloat16* out, cudaStream_t s) {
   const LayerSpec& L = kLayers[li];
   const DevLayer& dl = m->layers[li];
-  ConvArgs a;
-  a.src0 = src0; a.src1 = src1; a.C0 = dl.cfg.real0; a.C1 = dl.cfg.real1; a.Cin = a.C0 + a.C1;
-  a.P0 = c0; a.P1 = c1;
-  a.H0 = h0; a.W0 = w0; a.B = B; a.D = D; a.Hin = hin; a.Win = win;
-  a.stride = stride; a.ksize = L.k; a.pad = L.k / 2;
-  a.Hout = (hin + 2 * a.pad - L.k) / stride + 1;
-  a.Wout = (win + 2 * a.pad - L.k) / stride + 1;
-  a.taps = L.k * L.k * L.k;
-  a.num_kb = dl.num_kb;
-  a.M = B * D * a.Hout * a.Wout;
-  a.Cout = L.cout;
-  a.wpack = dl.wpack; a.scale = dl.scale; a.shift = dl.shift;
-  a.inv_sigma = dl.sn_index >= 0 ? m->inv_sigma_dev + dl.sn_index : nullptr;
-  a.residual = residual; a.out = out; a.act = act;
-  a.error_flag = m->error_flag_dev;
-  if (dl.cfg.kind != 1 || c0 != dl.cfg.real0 || c1 != dl.cfg.real1)
+  if (dl.cfg.kernel != Kernel::Gather || c0 != dl.cfg.real0 || c1 != dl.cfg.real1)
     return set_error(V2CE_ERR_STATE, "layer %s: gather launch with pitches %d+%d, expected %d+%d", L.name, c0, c1,
                      dl.cfg.real0, dl.cfg.real1);
-  return conv::launch_conv(a, dl.bn_tile, s);
+  return conv::launch_conv(conv_args(dl, L.k, L.cout, src0, c0, h0, w0, src1, c1, B, D, hin, win, stride, residual, act,
+                                     out, m->error_flag_dev),
+                           dl.bn_tile, s);
 }
 
 // halo-tile launch of layer `li` (3x3x3, stride 1); sources are full-resolution (B,D,H,W,pitch) tensors
@@ -622,46 +707,26 @@ static int run_halo(v2ce_model* m, int li, const __nv_bfloat16* src0, int p0, co
                     __nv_bfloat16* short_out = nullptr, int short_pitch = 0, bool* short_done = nullptr) {
   const LayerSpec& L = kLayers[li];
   const DevLayer& dl = m->layers[li];
-  if (dl.cfg.kind != 2 || p0 != dl.cfg.real0 || p1 != dl.cfg.real1)
+  if (dl.cfg.kernel != Kernel::Halo || p0 != dl.cfg.real0 || p1 != dl.cfg.real1)
     return set_error(V2CE_ERR_STATE, "layer %s: halo launch with pitches %d+%d, expected %d+%d", L.name, p0, p1,
                      dl.cfg.real0, dl.cfg.real1);
   const halo::HaloPlan plan = halo::plan_for(dl.bn_tile, D, H, W);
   // layers with few output channels: depth taps merged into the MMA N dimension (conv_halo_kdm.cuh)
   const halo::KdmPlan kplan = halo::plan_kdm(D, H, W);
   const bool kdm = dl.wpack_kdm != nullptr && kplan.ok;     // packed for Cout <= 64 (pack_layer)
-  halo::HaloArgs a;
-  a.a_row16 = 8; a.a_desc_hi = 0x40004040u;      // 64-channel SWIZZLE_128B patch rows
-  a.tap_mask = 0x1FF;
-  a.B = B; a.D = D; a.H = H; a.W = W;
-  a.PW = plan.ts.PW; a.TH = plan.ts.TH; a.TW = plan.ts.PW - 2;
-  a.tiles_w = (W + a.TW - 1) / a.TW;
-  a.tiles_h = (H + a.TH - 1) / a.TH;
-  a.ncc0 = dl.cfg.pad0 / 64; a.ncc1 = dl.cfg.pad1 / 64;
-  a.real0 = dl.cfg.real0; a.real1 = dl.cfg.real1;
-  a.Cout = L.cout; a.out_pitch = out_pitch; a.res_pitch = res_pitch;
-  a.T = plan.T; a.SA = plan.SA; a.SB = plan.SB; a.a_stage_bytes = plan.a_stage_bytes; a.box_bytes = plan.box_bytes;
-  a.wpack = dl.wpack; a.scale = dl.scale; a.shift = dl.shift;
-  if (kdm) { a.T = halo::kKdmT; a.SA = kplan.SA; a.SB = 9; a.wpack = dl.wpack_kdm; a.a_stage_bytes = kplan.a_stage_bytes; }
-  a.inv_sigma = dl.sn_index >= 0 ? m->inv_sigma_dev + dl.sn_index : nullptr;
-  a.residual = residual; a.out = out; a.act = act;
-  a.up_H = up_H; a.up_W = up_W;
-  a.pred_w = pred_out ? m->layers[kNumLayers - 1].w32 : nullptr;
-  a.pred_b = pred_out ? m->layers[kNumLayers - 1].bias : nullptr;
-  a.pred_out = pred_out;
-  a.error_flag = m->error_flag_dev;
+  const DevLayer& pred = m->layers[kNumLayers - 1];
+  const halo::HaloArgs a = halo_args(dl, View::Patch64, &plan, kdm ? &kplan : nullptr, B, D, H, W, L.cout, out, out_pitch,
+                                     residual, res_pitch, act, m->error_flag_dev, up_H, up_W, pred_out ? &pred : nullptr,
+                                     pred_out);
   if (pred_out) {
-    // constant memory is per device, not per handle: reload when another handle ran last (stream ordered)
     static unsigned long long pred_owner[64] = {0};
-    if (pred_owner[m->device & 63] != m->uid) {
-      if (int e = halo::load_pred_constants(a.pred_w, a.pred_b, s)) return e;
-      pred_owner[m->device & 63] = m->uid;
-    }
+    if (int e = load_constants(pred_owner, m, [&] { return halo::load_pred_constants(pred.w32, pred.bias, s); })) return e;
   }
   CUtensorMap tm0, tm1;
-  if (int e = get_tmap(m, src0, B, D, H, W, p0, a.PW, a.TH + 2, &tm0)) return e;
+  if (int e = get_tmap(m, MapKey{View::Patch64, 0, src0, B, D, H, W, p0, a.PW, a.TH + 2}, &tm0)) return e;
   tm1 = tm0;
   if (src1)
-    if (int e = get_tmap(m, src1, B, D, H, W, p1, a.PW, a.TH + 2, &tm1)) return e;
+    if (int e = get_tmap(m, MapKey{View::Patch64, 0, src1, B, D, H, W, p1, a.PW, a.TH + 2}, &tm1)) return e;
   if (short_done) *short_done = false;
   if (kdm) {
     // fuse the block's 1x1x1 shortcut conv (layer short_li) when asked for and packed
@@ -688,34 +753,11 @@ static int run_enc_kdm(v2ce_model* m, int li, const __nv_bfloat16* x, int pin, i
   const int Hout = (Hin - 1) / 2 + 1, Wout = (Win - 1) / 2 + 1;
   const halo::KdmPlan kp = halo::plan_kdm(D, Hout, Wout, 2);
   if (!kp.ok || dl.wpack_kdm == nullptr || sl.wpack_kdm == nullptr || Hin < 2 || Win < 2) return V2CE_OK;
-  halo::HaloArgs a;
-  a.a_row16 = 8; a.a_desc_hi = 0x40004040u;      // 64-channel SWIZZLE_128B patch rows
-  a.tap_mask = 0x1FF;
-  a.B = B; a.D = D; a.H = Hout; a.W = Wout;
-  a.PW = kp.ts.PW; a.TH = kp.ts.TH; a.TW = kp.TW;
-  a.tiles_w = (Wout + a.TW - 1) / a.TW;
-  a.tiles_h = (Hout + a.TH - 1) / a.TH;
-  a.ncc0 = chunk_of(dl.cfg.real0) / 64; a.ncc1 = 0;
-  a.real0 = dl.cfg.real0; a.real1 = 0;
-  a.Cout = L.cout; a.out_pitch = L.cout; a.res_pitch = 0;
-  a.T = halo::kKdmT; a.SA = kp.SA; a.SB = 9; a.a_stage_bytes = kp.a_stage_bytes; a.box_bytes = kp.box_bytes;
-  a.wpack = dl.wpack_kdm; a.scale = dl.scale; a.shift = dl.shift;
-  a.inv_sigma = nullptr;
-  a.residual = nullptr; a.out = out; a.act = 1;
-  a.up_H = 0; a.up_W = 0; a.pred_w = nullptr; a.pred_b = nullptr; a.pred_out = nullptr;
-  a.error_flag = m->error_flag_dev;
+  const halo::HaloArgs a = halo_args(dl, View::Parity, nullptr, &kp, B, D, Hout, Wout, L.cout, out, L.cout, nullptr, 0, 1,
+                                     m->error_flag_dev);
   halo::ParityMaps pm;
-  for (int q = 0; q < 4; ++q) {
-    // cached by (ptr, geometry); the parity rides in the "rows" key slot with an offset that cannot collide
-    auto key = std::make_tuple(static_cast<const void*>(x), B, D, Hin, Win, pin, a.PW, 1000 + q * 100 + a.TH);
-    auto it = m->tmaps.find(key);
-    if (it == m->tmaps.end()) {
-      CUtensorMap tm;
-      if (int e = halo::make_parity_map(&tm, x, B, D, Hin, Win, pin, q >> 1, q & 1, a.PW, a.TH + 1)) return e;
-      it = m->tmaps.emplace(key, tm).first;
-    }
-    pm.m[q] = it->second;
-  }
+  for (int q = 0; q < 4; ++q)
+    if (int e = get_tmap(m, MapKey{View::Parity, q, x, B, D, Hin, Win, pin, a.PW, a.TH + 1}, &pm.m[q])) return e;
   halo::KdmShort sc{sl.wpack_kdm, sl.scale, sl.shift, short_out, L.cout};
   *done = true;
   return halo::launch_halo_kdm(pm.m[0], pm.m[0], a, &sc, kp.smem_bytes, s, &pm);
@@ -724,12 +766,12 @@ static int run_enc_kdm(v2ce_model* m, int li, const __nv_bfloat16* x, int pin, i
 static int pack_layer(v2ce_model* m, int li, const float* w_dev, cudaStream_t s) {
   const LayerSpec& L = kLayers[li];
   DevLayer& dl = m->layers[li];
-  const LayerCfg c = layer_cfg(li);
+  const LayerCfg c = layer_cfg(L);
   dl.cfg = c;
   const int taps = L.k * L.k * L.k;
   const int cin_pad = c.pad0 + c.pad1;
   dl.bn_tile = conv::pick_bn(L.cout);
-  if (c.kind == 2 && L.cout == 256) {
+  if (c.kernel == Kernel::Halo && L.cout == 256) {
     // N tile of the 256- / 512-channel halo layers.  256-channel layers run as two N = 128 tiles: at 33 x 44 x 16 x 4
     // an N = 256 launch has 448 items = 3.03 waves of 148 CTAs (a quarter of the last wave's time is 4 items), the
     // N = 128 launch has 896 half-size items = 6.05 waves (3.5 full-item times) and a double-buffered accumulator, so
@@ -739,7 +781,7 @@ static int pack_layer(v2ce_model* m, int li, const float* w_dev, cudaStream_t s)
     dl.bn_tile = 128;
   }
   if (c.real0 + c.real1 != L.cin) return set_error(V2CE_ERR_STATE, "layer %s: channel split mismatch", L.name);
-  if (c.kind == 2) {
+  if (c.kernel == Kernel::Halo) {
     const size_t n = (size_t)L.cout * 27 * cin_pad;
     dl.num_kb = 27 * cin_pad / conv::kBlockK;
     if (int e = dev_alloc(m, &dl.wpack, n)) return e;
@@ -754,8 +796,7 @@ static int pack_layer(v2ce_model* m, int li, const float* w_dev, cudaStream_t s)
     }
     return V2CE_OK;
   }
-  const bool is_encoder = std::string(L.name).find("encoders") != std::string::npos;
-  if (is_encoder && L.k == 3 && std::string(L.name).find(".conv1") != std::string::npos) {
+  if (L.role == Role::EncConv1) {
     // stride-2 first conv of an encoder block: depth-merged packing for the parity-view kernel (conv_halo_kdm.cuh, S = 2)
     const size_t nk = (size_t)L.cout * 27 * chunk_of(c.real0);
     if (int e = dev_alloc(m, &dl.wpack_kdm, nk)) return e;
@@ -763,8 +804,8 @@ static int pack_layer(v2ce_model* m, int li, const float* w_dev, cudaStream_t s)
         w_dev, L.cout, L.cin, chunk_of(c.real0), c.real0, 0, 0, dl.wpack_kdm);
     V2CE_LAUNCH_CHECK("pack_weights_kdm_kernel");
   }
-  if (L.k == 1 && ((L.cout <= 64 && std::string(L.name).find("decoders") != std::string::npos) || is_encoder)) {
-    // the shortcut of a decoder block can ride in its conv1 launch (conv_halo_kdm.cuh): [Cout/32][cc][32][64]
+  if (L.role == Role::EncShort || (L.role == Role::DecShort && L.cout <= 64)) {
+    // the shortcut of an encoder or decoder block can ride in its conv1 launch (conv_halo_kdm.cuh): [Cout/32][cc][32][64]
     const int k0 = chunk_of(c.real0), k1 = c.real1 ? chunk_of(c.real1) : 0;
     const size_t ns = (size_t)L.cout * (k0 + k1);
     if (int e = dev_alloc(m, &dl.wpack_kdm, ns)) return e;
@@ -849,10 +890,9 @@ extern "C" int v2ce_model_finalize(v2ce_model* m) {
     if (int e = upload(m, &dl.w32, *w)) return e;
     const std::vector<float>* bias = L.bias ? find(m, base + ".bias") : nullptr;
     if (L.bias && (!bias || (int)bias->size() != L.cout)) return set_error(V2CE_ERR_STATE, "missing bias for %s", L.name);
-    const bool direct = (li == 0 || li == kNumLayers - 1);   // head and pred run on CUDA cores in fp32
-    if (direct) {
+    if (layer_cfg(L).kernel == Kernel::Direct) {   // head and pred run on CUDA cores in fp32
       if (int e = upload(m, &dl.bias, *bias)) return e;
-      if (li == 0) {
+      if (L.role == Role::Head) {
         if (int e = dev_alloc(m, &m->head_wpack, (size_t)27 * 2 * 32)) return e;
         pack_head_kernel<<<(27 * 2 * 32 + 255) / 256, 256, 0, s>>>(dl.w32, m->head_wpack);
         V2CE_LAUNCH_CHECK("pack_head_kernel");
@@ -891,7 +931,7 @@ extern "C" int v2ce_model_finalize(v2ce_model* m) {
     if (int e = pack_layer(m, li, dl.w32, s)) return e;
     if (L.sn) {
       V2CE_REQUIRE(sn_count < kNumSn, "too many spectral-norm layers");
-      dl.sn_index = sn_count;
+      dl.inv_sigma = m->inv_sigma_dev + sn_count;
       SnDesc& d = m->sn_descs_host[sn_count];
       d.rows = L.cout;
       d.K = L.cin * taps;
@@ -954,7 +994,6 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
   const Buffers buf = carve(ws_dev, d);
   if (buf.bytes > ws_bytes) return set_error(V2CE_ERR_WORKSPACE, "workspace too small: need %zu, got %zu", buf.bytes, ws_bytes);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  int launches = 0;
   size_t n_marks = 0;
   auto mark = [&](const char* what) {             // per-launch timing (tools/layer_times.py); off by default
     if (!m->layer_timing) return;
@@ -967,10 +1006,6 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     cudaEventRecord(m->marks[n_marks].second, s);
     ++n_marks;
   };
-  // option "stop_after": return right after the launch that writes layer stop_after's output (a block's shortcut fused
-  // into its conv1 stops there, pred stops after decoders.3.conv2), with the side stream joined into `s`.  Every launch
-  // writes out of place, so the workspace then holds both the inputs of that layer and its output.
-  auto stop_at = [&](int l0, int l1) { return m->stop_after >= 0 && (m->stop_after == l0 || m->stop_after == l1); };
   auto stop = [&]() -> int {
     V2CE_CUDA_CHECK(cudaEventRecord(m->ev_join, m->sn_stream));
     V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_join, 0));
@@ -982,7 +1017,16 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
   V2CE_CUDA_CHECK(cudaStreamWaitEvent(m->sn_stream, m->ev_fork, 0));
   if (int e = run_sn_step(m, m->sn_stream)) return e;
   V2CE_CUDA_CHECK(cudaEventRecord(m->ev_join, m->sn_stream));
-  launches += 4;
+  int launches = kSnLaunches;
+  // After the launch that writes layer li's output: count it, record the layer's timing mark, and tell whether the
+  // option "stop_after" ends the forward here -- at li, or at `also` (a block's shortcut fused into its conv1, pred in
+  // decoders.3.conv2).  The caller then returns stop(), with the side stream joined into `s`.  Every launch writes out
+  // of place, so the workspace then holds both the inputs of that layer and its output.
+  auto launched = [&](int li, int also = -1) {
+    ++launches;
+    mark(kLayers[li].name);
+    return m->stop_after >= 0 && (m->stop_after == li || m->stop_after == also);
+  };
 
   const long long M0 = d.M[0];
   // 32-byte patch rows: 16-channel SWIZZLE_32B view of the 8-channel split pixels
@@ -994,91 +1038,54 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     if (frames_u8) head_prep_kernel<true><<<pgrid, 256, 0, s>>>(x_dev, B, D, H, W, buf.head_in);
     else head_prep_kernel<false><<<pgrid, 256, 0, s>>>(x_dev, B, D, H, W, buf.head_in);
     V2CE_LAUNCH_CHECK("head_prep_kernel");
-    const DevLayer& dl = m->layers[0];
-    halo::HaloArgs a;
-  a.a_row16 = 8; a.a_desc_hi = 0x40004040u;      // 64-channel SWIZZLE_128B patch rows
-  a.tap_mask = 0x1FF;
-    a.B = B; a.D = D; a.H = H; a.W = W;
-    a.PW = hplan.ts.PW; a.TH = hplan.ts.TH; a.TW = hplan.TW;
-    a.tiles_w = (W + a.TW - 1) / a.TW;
-    a.tiles_h = (H + a.TH - 1) / a.TH;
-    a.ncc0 = 1; a.ncc1 = 0; a.real0 = 8; a.real1 = 0;
-    // taps (kh, 0) and (kh, 1): the kw = 2 weights ride in the upper half of kw = 1
-    a.tap_mask = 0x0DB;
-    a.Cout = 32; a.out_pitch = 32; a.res_pitch = 0;
-    a.T = halo::kKdmT; a.SA = hplan.SA; a.SB = 9; a.a_stage_bytes = hplan.a_stage_bytes; a.box_bytes = hplan.box_bytes;
-    a.wpack = dl.wpack_kdm; a.scale = dl.scale; a.shift = dl.shift; a.inv_sigma = nullptr;
-    a.residual = nullptr; a.out = buf.head; a.act = 2;
-    a.up_H = 0; a.up_W = 0; a.pred_w = nullptr; a.pred_b = nullptr; a.pred_out = nullptr;
-    a.error_flag = m->error_flag_dev;
-    CUtensorMap tmh;
-    {
-      a.a_row16 = 2; a.a_desc_hi = 0xC0004010u;     // K-major SWIZZLE_32B, 8-row groups 256 B apart
-      // cached like the other maps; pitch key 16 marks the 16-channel view of this pointer
-      auto key = std::make_tuple((const void*)buf.head_in, B, D, H, W, 16, a.PW, a.TH + 2);
-      auto it = m->tmaps.find(key);
-      if (it == m->tmaps.end()) {
-        CUtensorMap tm;
-        if (int e = halo::make_patch_map16(&tm, buf.head_in, B, D, H, W, a.PW, a.TH + 2)) return e;
-        it = m->tmaps.emplace(key, tm).first;
-      }
-      tmh = it->second;
-    }
-    if (int e = halo::launch_halo_kdm(tmh, tmh, a, nullptr, hplan.smem_bytes, s)) return e;
     ++launches;
+    const halo::HaloArgs a = halo_args(m->layers[0], View::Head16, nullptr, &hplan, B, D, H, W, 32, buf.head, 32, nullptr,
+                                       0, 2, m->error_flag_dev);
+    CUtensorMap tm;
+    if (int e = get_tmap(m, MapKey{View::Head16, 0, buf.head_in, B, D, H, W, 8, a.PW, a.TH + 2}, &tm)) return e;
+    if (int e = halo::launch_halo_kdm(tm, tm, a, nullptr, hplan.smem_bytes, s)) return e;
   } else {
     const long long groups = (long long)B * D * H * ((W + 3) / 4);
-    // constant memory is per device, not per handle: reload when another handle ran last (stream ordered)
     static unsigned long long head_owner[64] = {0};
-    if (head_owner[m->device & 63] != m->uid) {
-      V2CE_CUDA_CHECK(cudaMemcpyToSymbolAsync(c_head_w, m->head_wpack, sizeof(float) * 27 * 2 * 32, 0, cudaMemcpyDeviceToDevice, s));
-      V2CE_CUDA_CHECK(cudaMemcpyToSymbolAsync(c_head_b, m->layers[0].bias, sizeof(float) * 32, 0, cudaMemcpyDeviceToDevice, s));
-      head_owner[m->device & 63] = m->uid;
-    }
+    if (int e = load_constants(head_owner, m, [&]() -> int {
+          V2CE_CUDA_CHECK(cudaMemcpyToSymbolAsync(c_head_w, m->head_wpack, sizeof(float) * 27 * 2 * 32, 0, cudaMemcpyDeviceToDevice, s));
+          V2CE_CUDA_CHECK(cudaMemcpyToSymbolAsync(c_head_b, m->layers[0].bias, sizeof(float) * 32, 0, cudaMemcpyDeviceToDevice, s));
+          return V2CE_OK;
+        }))
+      return e;
     if (frames_u8)
       head_conv_kernel<true><<<(int)((groups + 127) / 128), 128, 0, s>>>(x_dev, B, D, H, W, buf.head);
     else
       head_conv_kernel<false><<<(int)((groups + 127) / 128), 128, 0, s>>>(x_dev, B, D, H, W, buf.head);
     V2CE_LAUNCH_CHECK("head_conv_kernel");
   }
-  ++launches;
-  mark("UNet.head.conv3d");
-  if (stop_at(0, -1)) return stop();
+  if (launched(0)) return stop();
 
   static const int ch[5] = {32, 64, 128, 256, 512};
-  char name[64];
   const __nv_bfloat16* x = buf.head;
   // encoders: conv1 and the shortcut are stride (1,2,2) -> gather kernel; conv2 -> halo kernel
   for (int i = 0; i < 4; ++i) {
-    snprintf(name, sizeof(name), "UNet.encoders.%d.conv1", i);
-    const int l1 = layer_index(name);
+    const int l1 = conv1_of(Role::EncConv1, i);
     const int pin = ch[i], co = ch[i + 1];
     bool fused = false;
     if (int e = run_enc_kdm(m, l1, x, pin, B, D, d.H[i], d.W[i], buf.tmp_t, buf.tmp_r, s, &fused)) return e;
     if (fused) {
-      mark(kLayers[l1].name);
-      launches -= 1;
-      if (stop_at(l1, l1 + 2)) return stop();
+      if (launched(l1, l1 + 2)) return stop();
     } else {
       if (int e = run_conv(m, l1, x, pin, d.H[i], d.W[i], nullptr, 0, B, D, d.H[i], d.W[i], 2, nullptr, 1, buf.tmp_t, s)) return e;
-      mark(kLayers[l1].name);
-      if (stop_at(l1, -1)) return stop();
+      if (launched(l1)) return stop();
       if (int e = run_conv(m, l1 + 2, x, pin, d.H[i], d.W[i], nullptr, 0, B, D, d.H[i], d.W[i], 2, nullptr, 0, buf.tmp_r, s)) return e;
-      mark(kLayers[l1 + 2].name);
-      if (stop_at(l1 + 2, -1)) return stop();
+      if (launched(l1 + 2)) return stop();
     }
     if (int e = run_halo(m, l1 + 1, buf.tmp_t, co, nullptr, 0, B, D, d.H[i + 1], d.W[i + 1], buf.tmp_r, co, 1, buf.enc[i], co, s)) return e;
-    mark(kLayers[l1 + 1].name);
-    if (stop_at(l1 + 1, -1)) return stop();
+    if (launched(l1 + 1)) return stop();
     x = buf.enc[i];
-    launches += 3;
   }
   // residual blocks at the bottleneck (first spectral-norm convs: join the side stream here)
   V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_join, 0));
   int side_ev = 0;
   for (int i = 0; i < 2; ++i) {
-    snprintf(name, sizeof(name), "UNet.resblocks.%d.conv1", i);
-    const int l1 = layer_index(name);
+    const int l1 = conv1_of(Role::ResConv1, i);
     // conv1 (persistent CTAs, a partial last wave) and the block's shortcut both read x: the shortcut goes to the
     // side stream AFTER conv1 so that its CTAs fill the SMs conv1 frees in its tail; conv2 waits for it.
     // (With per-launch timing on, everything stays on one stream.)
@@ -1088,17 +1095,15 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
       V2CE_CUDA_CHECK(cudaStreamWaitEvent(m->sn_stream, m->ev_side[side_ev], 0));
     }
     if (int e = run_halo(m, l1, x, 512, nullptr, 0, B, D, d.H[4], d.W[4], nullptr, 0, 1, buf.tmp_t, 512, s)) return e;
-    mark(kLayers[l1].name);
-    if (stop_at(l1, -1)) return stop();
+    if (launched(l1)) return stop();
     if (int e = run_conv(m, l1 + 2, x, 512, d.H[4], d.W[4], nullptr, 0, B, D, d.H[4], d.W[4], 1, nullptr, 0, buf.tmp_r,
                          side ? m->sn_stream : s)) return e;
-    mark(kLayers[l1 + 2].name);
     if (side) {
       V2CE_CUDA_CHECK(cudaEventRecord(m->ev_side[side_ev + 1], m->sn_stream));
       V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_side[side_ev + 1], 0));
       side_ev += 2;
     }
-    if (stop_at(l1 + 2, -1)) return stop();
+    if (launched(l1 + 2)) return stop();
     // the last block's output is only ever read nearest-upsampled by decoders.0: write it that way
     if (i == 1) {
       if (int e = run_halo(m, l1 + 1, buf.tmp_t, 512, nullptr, 0, B, D, d.H[4], d.W[4], buf.tmp_r, 512, 1, buf.up, 512, s,
@@ -1106,10 +1111,8 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     } else {
       if (int e = run_halo(m, l1 + 1, buf.tmp_t, 512, nullptr, 0, B, D, d.H[4], d.W[4], buf.tmp_r, 512, 1, buf.res[i], 512, s)) return e;
     }
-    mark(kLayers[l1 + 1].name);
-    if (stop_at(l1 + 1, -1)) return stop();
+    if (launched(l1 + 1)) return stop();
     x = buf.res[i];
-    launches += 3;
   }
   // decoders: virtual concat [nearest_up(x), skip]; skips are enc2, enc1, enc0, head.  `up` is written directly by
   // the epilogue of the layer that produced x (upsample-on-store); two buffers alternate because a decoder reads
@@ -1121,8 +1124,7 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     const int lvl = 3 - i;                       // output level
     const __nv_bfloat16* skip = lvl == 0 ? buf.head : buf.enc[lvl - 1];
     const int co = ch[lvl];                      // channels of the skip and of the outputs
-    snprintf(name, sizeof(name), "UNet.decoders.%d.conv1", i);
-    const int l1 = layer_index(name);
+    const int l1 = conv1_of(Role::DecConv1, i);
     bool short_done = false;
     const bool side = !m->layer_timing && side_ev + 2 <= 16;
     if (side) {
@@ -1131,18 +1133,15 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
     }
     if (int e = run_halo(m, l1, up_cur, xc, skip, co, B, D, d.H[lvl], d.W[lvl], nullptr, 0, 1, buf.tmp_t, co, s, 0, 0, nullptr,
                          l1 + 2, buf.tmp_r, co, &short_done)) return e;
-    mark(kLayers[l1].name);
-    if (stop_at(l1, short_done ? l1 + 2 : -1)) return stop();
+    if (launched(l1, short_done ? l1 + 2 : -1)) return stop();
     if (!short_done) {
       if (int e = run_conv(m, l1 + 2, up_cur, xc, d.H[lvl], d.W[lvl], skip, co, B, D, d.H[lvl], d.W[lvl], 1, nullptr, 0, buf.tmp_r,
                            side ? m->sn_stream : s)) return e;
-      mark(kLayers[l1 + 2].name);
-      ++launches;
       if (side) {
         V2CE_CUDA_CHECK(cudaEventRecord(m->ev_side[side_ev + 1], m->sn_stream));
         V2CE_CUDA_CHECK(cudaStreamWaitEvent(s, m->ev_side[side_ev + 1], 0));
       }
-      if (stop_at(l1 + 2, -1)) return stop();
+      if (launched(l1 + 2)) return stop();
     }
     if (side) side_ev += 2;
     if (lvl > 0) {
@@ -1152,11 +1151,9 @@ static int forward_impl(v2ce_model* m, const void* x_dev, bool frames_u8, float*
       if (int e = run_halo(m, l1 + 1, buf.tmp_t, co, nullptr, 0, B, D, d.H[lvl], d.W[lvl], buf.tmp_r, co, 1, buf.dec[i], co, s,
                            0, 0, y_dev)) return e;
     }
-    mark(kLayers[l1 + 1].name);
-    if (stop_at(l1 + 1, lvl == 0 ? kNumLayers - 1 : -1)) return stop();
+    if (launched(l1 + 1, lvl == 0 ? kNumLayers - 1 : -1)) return stop();
     __nv_bfloat16* tsw = up_cur; up_cur = up_next; up_next = tsw;
     xc = co;
-    launches += 2;
   }
   m->last_launches = launches;
   return V2CE_OK;
@@ -1219,7 +1216,6 @@ extern "C" int v2ce_model_layer_times(v2ce_model* m, int32_t cap, float* ms_out,
 
 extern "C" int v2ce_model_set_option(v2ce_model* m, const char* key, int64_t value) {
   V2CE_REQUIRE(m && key, "NULL argument");
-  if (std::string(key) == "desc_mode") { m->desc_mode = (int)value; return V2CE_OK; }
   if (std::string(key) == "layer_timing") { m->layer_timing = (int)value; return V2CE_OK; }
   if (std::string(key) == "stop_after") {
     V2CE_REQUIRE(value >= -1 && value < kNumLayers, "stop_after must be -1 or a layer index < %d", kNumLayers);
@@ -1232,8 +1228,7 @@ extern "C" int v2ce_model_set_option(v2ce_model* m, const char* key, int64_t val
 extern "C" int v2ce_conv3d_bf16_ex(const void* src0_dev, int32_t c0, int32_t h0, int32_t w0, const void* src1_dev, int32_t c1,
                                    int32_t batch, int32_t depth, int32_t hin, int32_t win, int32_t ksize, int32_t stride_hw,
                                    const float* weight_host, int32_t cout, const float* scale_host, const float* shift_host,
-                                   const void* residual_dev, int32_t act, void* out_dev, int32_t impl, int32_t desc_mode,
-                                   void* stream) {
+                                   const void* residual_dev, int32_t act, void* out_dev, int32_t impl, void* stream) {
   V2CE_REQUIRE(src0_dev && weight_host && scale_host && shift_host && out_dev, "NULL argument");
   V2CE_REQUIRE(ksize == 1 || ksize == 3, "ksize must be 1 or 3");
   V2CE_REQUIRE(stride_hw == 1 || stride_hw == 2, "stride must be 1 or 2");
@@ -1276,42 +1271,34 @@ extern "C" int v2ce_conv3d_bf16_ex(const void* src0_dev, int32_t c0, int32_t h0,
   if (cudaGetLastError() != cudaSuccess) rc = set_error(V2CE_ERR_CUDA, "weight pack launch failed");
   const int pad = ksize / 2;
   const int hout = (hin + 2 * pad - ksize) / stride_hw + 1, wout = (win + 2 * pad - ksize) / stride_hw + 1;
+  // the hook's conv as a model layer whose channel pitches are its channel counts
+  DevLayer dl;
+  dl.cfg = LayerCfg{impl >= 1 ? Kernel::Halo : Kernel::Gather, c0, c0, c1, c1};
+  dl.wpack = dl.wpack_kdm = wpack;
+  dl.scale = scale_dev; dl.shift = shift_dev;
+  dl.bn_tile = bn; dl.num_kb = num_kb;
+  const __nv_bfloat16* src0 = static_cast<const __nv_bfloat16*>(src0_dev);
+  const __nv_bfloat16* src1 = static_cast<const __nv_bfloat16*>(src1_dev);
+  const __nv_bfloat16* residual = static_cast<const __nv_bfloat16*>(residual_dev);
+  __nv_bfloat16* out = static_cast<__nv_bfloat16*>(out_dev);
   if (rc == V2CE_OK && impl >= 1) {
     const halo::HaloPlan plan = halo::plan_for(bn, depth, hin, win);
     const halo::KdmPlan kplan = halo::plan_kdm(depth, hout, wout, stride_hw);
-    halo::HaloArgs a;
-  a.a_row16 = 8; a.a_desc_hi = 0x40004040u;      // 64-channel SWIZZLE_128B patch rows
-  a.tap_mask = 0x1FF;
-    a.B = batch; a.D = depth; a.H = hin; a.W = win;
-    a.PW = plan.ts.PW; a.TH = plan.ts.TH; a.TW = plan.ts.PW - 2;
-    a.tiles_w = (win + a.TW - 1) / a.TW; a.tiles_h = (hin + a.TH - 1) / a.TH;
-    a.ncc0 = c0 / 64; a.ncc1 = c1 / 64;
-    a.real0 = c0; a.real1 = c1;
-    a.Cout = cout; a.out_pitch = cout; a.res_pitch = cout;
-    a.T = plan.T; a.SA = plan.SA; a.SB = plan.SB; a.a_stage_bytes = plan.a_stage_bytes; a.box_bytes = plan.box_bytes;
-    a.wpack = wpack; a.scale = scale_dev; a.shift = shift_dev; a.inv_sigma = nullptr;
+    const bool s2 = stride_hw == 2;              // depth-merged variant only (checked above)
+    const halo::HaloArgs a = halo_args(dl, s2 ? View::Parity : View::Patch64, &plan, impl >= 2 ? &kplan : nullptr, batch,
+                                       depth, hout, wout, cout, out, cout, impl == 3 ? nullptr : residual, cout, act, flag);
     halo::ParityMaps pmaps;
-    const bool s2 = impl >= 2 && stride_hw == 2;
-    if (impl >= 2) {
-      a.T = halo::kKdmT; a.SA = kplan.SA; a.SB = 9; a.a_stage_bytes = kplan.a_stage_bytes; a.box_bytes = kplan.box_bytes;
-      a.H = hout; a.W = wout;
-      a.PW = kplan.ts.PW; a.TH = kplan.ts.TH; a.TW = kplan.TW;
-      a.tiles_w = (wout + a.TW - 1) / a.TW; a.tiles_h = (hout + a.TH - 1) / a.TH;
-    }
-    a.residual = impl == 3 ? nullptr : static_cast<const __nv_bfloat16*>(residual_dev);
-    a.out = static_cast<__nv_bfloat16*>(out_dev);
-    a.act = act; a.error_flag = flag;
-    a.up_H = 0; a.up_W = 0; a.pred_w = nullptr; a.pred_b = nullptr; a.pred_out = nullptr;
     CUtensorMap tm0, tm1;
     if (s2) {
       for (int q = 0; q < 4 && rc == V2CE_OK; ++q)
-        rc = halo::make_parity_map(&pmaps.m[q], src0_dev, batch, depth, hin, win, c0, q >> 1, q & 1, a.PW, a.TH + 1);
+        rc = make_map(MapKey{View::Parity, q, src0, batch, depth, hin, win, c0, a.PW, a.TH + 1}, &pmaps.m[q]);
       tm0 = pmaps.m[0];
     } else {
-      rc = halo::make_patch_map(&tm0, src0_dev, batch, depth, hin, win, c0, a.PW, a.TH + 2);
+      rc = make_map(MapKey{View::Patch64, 0, src0, batch, depth, hin, win, c0, a.PW, a.TH + 2}, &tm0);
     }
     tm1 = tm0;
-    if (rc == V2CE_OK && src1_dev) rc = halo::make_patch_map(&tm1, src1_dev, batch, depth, hin, win, c1, a.PW, a.TH + 2);
+    if (rc == V2CE_OK && src1)
+      rc = make_map(MapKey{View::Patch64, 0, src1, batch, depth, hin, win, c1, a.PW, a.TH + 2}, &tm1);
     if (rc == V2CE_OK && impl == 3) {
       // fused shortcut: 1x1x1 weights = centre tap of `weight`, same scale/shift, no activation -> residual_dev
       std::vector<float> wd((size_t)cout * cin);
@@ -1334,20 +1321,9 @@ extern "C" int v2ce_conv3d_bf16_ex(const void* src0_dev, int32_t c0, int32_t h0,
                      : halo::launch_halo(tm0, tm1, a, bn, plan.smem_bytes, s);
     }
   } else if (rc == V2CE_OK) {
-    ConvArgs a;
-    a.src0 = static_cast<const __nv_bfloat16*>(src0_dev);
-    a.src1 = static_cast<const __nv_bfloat16*>(src1_dev);
-    a.C0 = c0; a.C1 = c1; a.Cin = cin; a.P0 = c0; a.P1 = c1; a.H0 = h0; a.W0 = w0;
-    a.B = batch; a.D = depth; a.Hin = hin; a.Win = win;
-    a.stride = stride_hw; a.ksize = ksize; a.pad = pad;
-    a.Hout = hout; a.Wout = wout;
-    a.taps = taps; a.num_kb = num_kb;
-    a.M = batch * depth * hout * wout;
-    a.Cout = cout; a.wpack = wpack; a.scale = scale_dev; a.shift = shift_dev; a.inv_sigma = nullptr;
-    a.residual = static_cast<const __nv_bfloat16*>(residual_dev);
-    a.out = static_cast<__nv_bfloat16*>(out_dev);
-    a.act = act; a.error_flag = flag;
-    rc = conv::launch_conv(a, bn, s);
+    rc = conv::launch_conv(conv_args(dl, ksize, cout, src0, c0, h0, w0, src1, c1, batch, depth, hin, win, stride_hw, residual,
+                                     act, out, flag),
+                           bn, s);
   }
   cudaError_t se = cudaStreamSynchronize(s);
   int hflag = 0;
@@ -1357,14 +1333,6 @@ extern "C" int v2ce_conv3d_bf16_ex(const void* src0_dev, int32_t c0, int32_t h0,
   if (se != cudaSuccess) return set_error(V2CE_ERR_CUDA, "conv3d_bf16 failed: %s", cudaGetErrorString(se));
   if (hflag) return set_error(V2CE_ERR_CUDA, "conv pipeline watchdog fired");
   return V2CE_OK;
-}
-
-extern "C" int v2ce_conv3d_bf16(const void* src0_dev, int32_t c0, int32_t h0, int32_t w0, const void* src1_dev, int32_t c1,
-                                int32_t batch, int32_t depth, int32_t hin, int32_t win, int32_t ksize, int32_t stride_hw,
-                                const float* weight_host, int32_t cout, const float* scale_host, const float* shift_host,
-                                const void* residual_dev, int32_t act, void* out_dev, void* stream) {
-  return v2ce_conv3d_bf16_ex(src0_dev, c0, h0, w0, src1_dev, c1, batch, depth, hin, win, ksize, stride_hw, weight_host, cout,
-                             scale_host, shift_host, residual_dev, act, out_dev, 0, 0, stream);
 }
 
 // ------------------------------------------------------------------------------------------
