@@ -162,6 +162,19 @@ int v2ce_ts_diff_metric(const uint8_t* gt_records_dev, int64_t n_gt, const uint8
                         int32_t width, int32_t height, int32_t search_range, double cap_us, void* ws_dev, size_t ws_bytes,
                         int64_t* result_dev, void* stream);
 
+/* ---- event stream -> voxel grid (stage-2 evaluation inputs) -------------------------------------------------------
+ * The toolbox's own binning convention, not a port of the reference's training voxeliser.  Counts n_events packed
+ * 13-byte records (any order) into voxels_dev, float32 (F, 2, nbins, H, W), which the call overwrites (n_events = 0
+ * writes zeros).  Per record: x or y outside the width x height sensor -> status[0]; polarity 1 -> plane 0, 0 or -1 ->
+ * plane 1, any other value -> status[1]; t < frame_edges[0] -> status[2]; t >= frame_edges[F] -> status[3]; else frame f
+ * with edges[f] <= t < edges[f+1], L = edges[f+1] - edges[f], r = t - edges[f], bin c = ((r + 1) * nbins - 1) / L in
+ * int64 (bin c starts at edges[f] + floor(c * L / nbins)), and voxels[f, plane, c, y, x] += 1.  Counts are exact while a
+ * cell stays below 2^24, and then independent of the record order.
+ * frame_edges_us_dev: int64[F + 1], strictly increasing, every L * nbins < 2^62 (not checked on the device).
+ * status_dev: int64[4] = {outside the sensor, polarity not in {-1,0,1}, before frame_edges[0], at or after frame_edges[F]} */
+int v2ce_events_to_voxels(const uint8_t* records_dev, int64_t n_events, const int64_t* frame_edges_us_dev,
+                          int32_t n_frames, int32_t nbins, int32_t height, int32_t width,
+                          float* voxels_dev, int64_t* status_dev, void* stream);
 
 
 /* ------------------------------------------------------------------------------------------

@@ -63,6 +63,8 @@ _SIGNATURES = {
     'v2ce_ts_diff_workspace_bytes': (c_int, [c_int32, c_int32, c_int64, POINTER(c_size_t)]),
     'v2ce_ts_diff_metric': (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32, c_int32, c_double, c_void_p,
                                     c_size_t, c_void_p, c_void_p]),
+    'v2ce_events_to_voxels': (c_int, [c_void_p, c_int64, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p,
+                                      c_void_p]),
     'v2ce_peer_window_alloc': (c_int, [c_size_t, POINTER(c_void_p), c_void_p]),
     'v2ce_peer_window_free': (c_int, [c_void_p]),
     'v2ce_peer_window_open': (c_int, [c_void_p, POINTER(c_void_p)]),

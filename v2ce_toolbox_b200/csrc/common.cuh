@@ -51,6 +51,24 @@ struct Arena {
   bool ok() const { return off <= size; }
 };
 
+// One packed 13-byte event record (timestamp <i8, x <i2, y <i2, polarity i1; any alignment), as the LDATI and baseline
+// emitters write it.  Polarity -1 is folded into 0: the stage-2 metric (stage2_metrics.py:38-41) and the voxeliser
+// both treat -1 like 0.  Other polarity values are returned as they are, for the caller to reject.
+struct Rec { long long ts; int x, y, p; };
+
+__device__ __forceinline__ Rec load_rec(const uint8_t* __restrict__ r) {
+  unsigned long long t = 0ull;
+#pragma unroll
+  for (int b = 0; b < 8; ++b) t |= (unsigned long long)r[b] << (8 * b);
+  Rec e;
+  e.ts = (long long)t;
+  e.x = (int)(short)((unsigned)r[8] | ((unsigned)r[9] << 8));
+  e.y = (int)(short)((unsigned)r[10] | ((unsigned)r[11] << 8));
+  e.p = (int)(signed char)r[12];
+  if (e.p == -1) e.p = 0;
+  return e;
+}
+
 int sm_count_cached();
 // index (< 64) of the current CUDA device: function attributes and constant memory are per device, so the
 // one-time-setup caches of the launchers are kept per device (one process may drive several GPUs)

@@ -13,21 +13,6 @@
 namespace v2ce {
 namespace metrics {
 
-struct Rec { long long ts; int x, y, p; };
-
-__device__ __forceinline__ Rec load_rec(const uint8_t* __restrict__ r) {
-  unsigned long long t = 0ull;
-#pragma unroll
-  for (int b = 0; b < 8; ++b) t |= (unsigned long long)r[b] << (8 * b);
-  Rec e;
-  e.ts = (long long)t;
-  e.x = (int)(short)((unsigned)r[8] | ((unsigned)r[9] << 8));
-  e.y = (int)(short)((unsigned)r[10] | ((unsigned)r[11] << 8));
-  e.p = (int)(signed char)r[12];
-  if (e.p == -1) e.p = 0;                              // stage2_metrics.py:38-41
-  return e;
-}
-
 __global__ void cell_count_kernel(const uint8_t* __restrict__ pred, long long n, int W, int H, int* __restrict__ count,
                                   int* __restrict__ bad) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

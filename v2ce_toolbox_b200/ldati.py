@@ -186,6 +186,24 @@ def check_status(status_host):
                         f'(non-finite or out-of-contract voxel values)')
 
 
+def records_dev(ev, device):
+    """Packed 13-byte records on `device` and their count.  `ev`: a uint8 CUDA tensor of packed records (used as it
+    is) or a host record array with the fields timestamp, x, y, polarity of any integer widths (converted to
+    EVENT_DTYPE, then uploaded)."""
+    if isinstance(ev, torch.Tensor):
+        if not ev.is_cuda or ev.dtype != torch.uint8 or ev.numel() % 13:
+            raise V2ceError('event tensors must be uint8 CUDA tensors of packed 13-byte records')
+        return ev.contiguous().reshape(-1), ev.numel() // 13
+    ev = np.asarray(ev)
+    if ev.dtype != EVENT_DTYPE:
+        rec = np.empty(ev.shape[0], dtype=EVENT_DTYPE)
+        for f in ('timestamp', 'x', 'y', 'polarity'):
+            rec[f] = ev[f]
+        ev = rec
+    flat = torch.from_numpy(np.ascontiguousarray(ev).view(np.uint8).reshape(-1))
+    return flat.to(device), ev.shape[0]
+
+
 def split_frames(events_host, seg_counts_host):
     """events_host: uint8 (total*13,) host array -> list of per-frame recarrays (views)."""
     rec = events_host.view(EVENT_DTYPE)

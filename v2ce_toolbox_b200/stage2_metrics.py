@@ -15,22 +15,7 @@ import torch
 
 from . import _lib
 from ._lib import V2ceError, check, ptr, stream_ptr
-from .ldati import EVENT_DTYPE
-
-
-def _records_dev(ev, device):
-    if isinstance(ev, torch.Tensor):
-        if not ev.is_cuda or ev.dtype != torch.uint8 or ev.numel() % 13:
-            raise V2ceError('event tensors must be uint8 CUDA tensors of packed 13-byte records')
-        return ev.contiguous().reshape(-1), ev.numel() // 13
-    ev = np.asarray(ev)
-    if ev.dtype != EVENT_DTYPE:
-        rec = np.empty(ev.shape[0], dtype=EVENT_DTYPE)
-        for f in ('timestamp', 'x', 'y', 'polarity'):
-            rec[f] = ev[f]
-        ev = rec
-    flat = torch.from_numpy(np.ascontiguousarray(ev).view(np.uint8).reshape(-1))
-    return flat.to(device), ev.shape[0]
+from .ldati import records_dev as _records_dev
 
 
 def ts_diff_metric(event_gt, event_pred, search_range=0, fps=30, *, width=346, height=260, device=None):
