@@ -206,6 +206,21 @@ int v2ce_image_units(const uint8_t* frames_dev, int32_t n_windows, int32_t frame
                      int32_t src_w, int32_t dst_h, int32_t dst_w, float* units_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Window assembly for frames that arrive one by one (v2ce_toolbox_b200/clip_stream.py): writes the uint8 gray windows
+ * of one batch, out_dev (n_windows, frames_per_window, height, out_width), from source frames that stay where they are.
+ *   frames_dev: int64[2 * n_src] = {frame address, row pitch in bytes} per source frame; a frame is height rows of
+ *               width pixels of `channels` consecutive bytes (a row-cropped view or an (H, W, C) channels-last tensor)
+ *   slots_dev:  int32[n_windows * frames_per_window], the source frame of each output frame (windows may share frames)
+ *   channels 1 = gray (copied), 3 / 4 = colour with alpha ignored, converted like OpenCV's cvtColor(*2GRAY) for 8-bit
+ *   input: gray = (3735 * B + 19235 * G + 9798 * R + 2^14) >> 15; rgb_order 0 = B first (BGR, BGRA), 1 = R first.
+ *   Output column x reads source column x0 + x: x0 = width / 2 - out_width / 2 is the center crop of v2ce.py:78.
+ * Slots and frame addresses are not checked on the device.
+ * ------------------------------------------------------------------------------------------ */
+int v2ce_assemble_windows(const int64_t* frames_dev, const int32_t* slots_dev, int32_t n_windows,
+                          int32_t frames_per_window, int32_t height, int32_t width, int32_t channels,
+                          int32_t rgb_order, int32_t x0, int32_t out_width, uint8_t* out_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Stage 1 -- V2ce3d.  Replaces scripts/v2ce_3d.py:12-30 (V2ce3d), scripts/unet_2layer.py:203-379
  * (UNet3D), scripts/submodules.py:85-124,216-264 (ConvLayer3D, ResidualBlock3D) and
  * scripts/spectral_norm.py:9-64 (SpectralNorm) in eval mode.

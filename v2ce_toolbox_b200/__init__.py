@@ -6,6 +6,7 @@ device computation is hand-written CUDA in libv2ce_b200.so, reached through the 
 include/v2ce_b200.h.  No CPU fallback: CPU tensors and a missing library raise.
 """
 from ._lib import V2ceError, load  # noqa: F401
+from .clip_stream import ClipStream  # noqa: F401
 from .voxelize import events_to_voxels  # noqa: F401
 
 __version__ = '0.1.0'

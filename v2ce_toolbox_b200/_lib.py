@@ -75,6 +75,8 @@ _SIGNATURES = {
     'v2ce_ef_select': (c_int, [c_void_p, c_int64, c_double, c_int32, c_void_p, c_size_t, c_void_p, c_void_p]),
     'v2ce_ef_normalize': (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_double, c_void_p, c_void_p]),
     'v2ce_image_units': (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
+    'v2ce_assemble_windows': (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32,
+                                      c_int32, c_void_p, c_void_p]),
     'v2ce_model_create': (c_int, [POINTER(c_void_p), c_int]),
     'v2ce_model_destroy': (c_int, [c_void_p]),
     'v2ce_model_set_tensor': (c_int, [c_void_p, c_char_p, c_void_p, POINTER(c_int64), c_int32]),

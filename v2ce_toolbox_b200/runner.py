@@ -52,7 +52,7 @@ def nvtx(name):
 class Ticket:
     __slots__ = ('slot', 'n_pairs', 'total', 'seg_counts', 'done', 'status', 'ub', 'h2d_bytes', 'd2h_bytes', 'hw',
                  'pair_base', 'vox', 'sums', 'small_host', 'counts_ready', 'staged', 'params', 'offs', 'fwd_events',
-                 'events_dev', 'frames_dev', 'packed', 'ev_host')
+                 'events_dev', 'frames_dev', 'packed', 'ev_host', 'events_out')
 
 
 class BatchRunner:
@@ -76,6 +76,9 @@ class BatchRunner:
         self.host_sink = None
         self._all_ev = None
         self._all_bytes = 0
+        # True: every batch's packed events are also copied into a tensor of their own (Ticket.events_out), which later
+        # batches do not overwrite when they reuse the slot (clip_stream.ClipStream hands them out per batch)
+        self.events_out = False
         self.clip_pairs = 0                     # pairs of the clip being collected (v2ce.stream_clip sets it): sizes
         self._pairs_collected = 0               # the clip-wide buffer after the first batch instead of regrowing it
         self.lib = _lib.load()
@@ -276,6 +279,7 @@ class BatchRunner:
                     self._all_ev = grown
                 self._all_ev[self._all_bytes:need].copy_(ev[:total * 13])
                 self._all_bytes = need
+            t.events_out = ev[:total * 13].clone() if self.events_out else None
             t.ev_host = None
             if self.copy_out:
                 if self.host_sink is not None:

@@ -72,6 +72,14 @@ def window_schedule(frame_count, seq_len=16):
     return starts, mode
 
 
+def batch_plan(starts, mode, batch_size):
+    """v2ce.py:158-176 batching of the windows `starts`: [(first window, end window, trim_last_window_to)], `batch_size`
+    consecutive windows per model call; the batch holding the last window keeps only the last `mode` pairs of it
+    (v2ce.py:227-236, BatchRunner.submit)."""
+    n = len(starts)
+    return [(a, min(a + batch_size, n), mode if a + batch_size >= n else 0) for a in range(0, n, batch_size)]
+
+
 def pano_tiles(total_width, width=346):
     """v2ce.py:103-111 -- (src_start, src_end, columns kept from the right) per 346-px tile."""
     n = int(np.ceil(total_width / width))
@@ -228,13 +236,10 @@ def _batches(image_paths, vidcap, seq_len, height, batch_size, schedule=None):
     frame_count = vidcap.frame_count if vidcap is not None else len(image_paths)
     starts, mode = schedule if schedule is not None else window_schedule(frame_count, seq_len)
     read, close = _window_reader(image_paths, vidcap, starts, seq_len)
-    pending = []
     try:
-        for i in range(len(starts)):
-            pending.append(image_pre_processing(read(i), height)[None])
-            if len(pending) == batch_size or i == len(starts) - 1:
-                yield (torch.cat(pending, dim=0) if len(pending) > 1 else pending[0]), i == len(starts) - 1
-                pending = []
+        for a, e, _trim in batch_plan(starts, mode, batch_size):
+            pending = [image_pre_processing(read(i), height)[None] for i in range(a, e)]
+            yield (torch.cat(pending, dim=0) if len(pending) > 1 else pending[0]), e == len(starts)
     finally:
         close()
 
@@ -295,28 +300,100 @@ def _window_batches_u8(image_paths, vidcap, seq_len, batch_size, schedule, width
     """Raw uint8 windows in the reference's batching: (b, L+1, H, width) center-cropped like v2ce.py:78, or the whole
     frames (b, L+1, H, W) when `width` is None (the device then resizes them, preprocess.image_units_device)."""
     frame_count = vidcap.frame_count if vidcap is not None else len(image_paths)
-    starts, _ = schedule if schedule is not None else window_schedule(frame_count, seq_len)
+    starts, mode = schedule if schedule is not None else window_schedule(frame_count, seq_len)
     read, close = _window_reader(image_paths, vidcap, starts, seq_len)
-    pending = []
     pin = torch.cuda.is_available()
     try:
-        for i in range(len(starts)):
-            fr = np.asarray(read(i))
-            if width is not None:
-                c = fr.shape[-1] // 2
-                fr = fr[..., c - width // 2:c + width // 2]
-            pending.append(fr)
-            if len(pending) == batch_size or i == len(starts) - 1:
-                # ONE copy per frame, straight into the page-locked batch the H2D transfer reads (a 1080p window is
-                # 35 MB: stacking, concatenating and pinning it separately made the host the bottleneck of a pano clip)
-                out = torch.empty((len(pending),) + tuple(pending[0].shape), dtype=torch.uint8, pin_memory=pin)
-                o = out.numpy()
-                for j, w in enumerate(pending):
-                    np.copyto(o[j], w)
-                yield out, i == len(starts) - 1
-                pending = []
+        for a, e, _trim in batch_plan(starts, mode, batch_size):
+            pending = []
+            for i in range(a, e):
+                fr = np.asarray(read(i))
+                if width is not None:
+                    c = fr.shape[-1] // 2
+                    fr = fr[..., c - width // 2:c + width // 2]
+                pending.append(fr)
+            # ONE copy per frame, straight into the page-locked batch the H2D transfer reads (a 1080p window is
+            # 35 MB: stacking, concatenating and pinning it separately made the host the bottleneck of a pano clip)
+            out = torch.empty((len(pending),) + tuple(pending[0].shape), dtype=torch.uint8, pin_memory=pin)
+            o = out.numpy()
+            for j, w in enumerate(pending):
+                np.copyto(o[j], w)
+            yield out, e == len(starts)
     finally:
         close()
+
+
+def _frame_route(model, infer_type, dtype, shape, height, width, device_resize, pano=_pano_device):
+    """How the gray frames of a clip, `shape` (..., H, W), reach the model: ('native', None) when they already have the
+    model's resolution (raw uint8 windows, center-cropped, go to forward_frames; the resize of image_pre_processing is
+    the identity and the rest of it runs inside the head conv); ('raw', infer) for uint8 frames at another resolution
+    (whole uint8 windows are uploaded; /255, the cv2-exact bilinear resize, pair stacking and Normalize run in one
+    kernel, preprocess.image_units_device, bit-identical to the host path -- SURVEY.md N1); (None, None) otherwise
+    (float image units from the host)."""
+    H, W = shape[-2], shape[-1]
+    if (infer_type == 'center' and hasattr(model, 'forward_frames') and dtype == np.uint8 and H == height and
+            int(W / H * height) == W and W >= width and width % 2 == 0):
+        return 'native', None
+    if device_resize and dtype == np.uint8 and len(shape) == 3 and H >= 2:
+        from .preprocess import image_units_device
+        tile = _center_device if infer_type == 'center' else pano
+        return 'raw', (lambda u8: tile(model, image_units_device(u8, height), width))
+    return None, None
+
+
+def _claim_model(model):
+    """One clip at a time per model: the spectral-norm state advances per model call, so two interleaved clips would
+    each change the other's sigma, and they would share the model's BatchRunner."""
+    if model.__dict__.get('_v2ce_clip_open'):
+        raise RuntimeError('this model is already converting a clip (a ClipStream that has not been closed)')
+    model.__dict__['_v2ce_clip_open'] = True
+
+
+def _release_model(model):
+    model.__dict__['_v2ce_clip_open'] = False
+
+
+class _ClipRun:
+    """The device half of one clip, shared by stream_clip and clip_stream.ClipStream: the model's BatchRunner, the pair
+    index each batch starts at, and the clip-global event frames (v2ce.py:262-264) over the per-pair sums.
+    hand_out=False collects the events of every batch in one device buffer (runner.collected_events); True gives each
+    batch's events a tensor of its own (Ticket.events_out)."""
+
+    def __init__(self, model, device, infer, fps, ceil, percentile, keep_polarity, seed, pair_base, keep_sums,
+                 hand_out, clip_pairs=0):
+        from .runner import BatchRunner
+        # the runner owns ~0.5 GB of pinned staging buffers whose allocation costs more than a short clip's compute:
+        # one per (model, device), reused across calls
+        cache = model.__dict__.setdefault('_v2ce_runners', {})
+        runner = cache.get(str(device))
+        if runner is None:
+            runner = cache[str(device)] = BatchRunner(model, device, per_batch_frames=False, copy_out=False,
+                                                      collect_on_device=True)
+        runner.fps, runner.ceil, runner.percentile, runner.keep, runner.seed = fps, ceil, percentile, keep_polarity, seed
+        runner.infer = infer
+        runner.collect_on_device, runner.events_out = not hand_out, hand_out
+        runner.sums = []
+        runner.reset_collection()
+        runner.clip_pairs = clip_pairs
+        self.runner, self.device, self.keep_sums = runner, device, keep_sums
+        self.percentile, self.ceil, self.keep = percentile, ceil, keep_polarity
+        self.pair_idx = pair_base
+
+    def submit(self, x, trim_last_window_to):
+        t = self.runner.submit(x, self.pair_idx, keep_sums=self.keep_sums, trim_last_window_to=trim_last_window_to)
+        self.pair_idx += t.n_pairs
+        return t
+
+    def event_frames(self, write_event_frames):
+        """(uint8 BGR preview frames | None, upper bound | None, per-pair sums | None) once every batch is submitted."""
+        frames, ub, sums = None, None, None
+        if self.keep_sums:
+            torch.cuda.current_stream(self.device).wait_stream(self.runner.post_stream)
+            sums = torch.cat(self.runner.sums, dim=0) if len(self.runner.sums) > 1 else self.runner.sums[0]
+        if write_event_frames:
+            ub = _ef.upper_bound(sums, self.percentile, self.ceil, self.keep)
+            frames = _ef.normalize(sums, ub, self.keep).cpu().numpy()
+        return frames, ub, sums
 
 
 @torch.no_grad()
@@ -328,7 +405,6 @@ def stream_clip(model, image_paths=None, vidcap=None, infer_type='center', seq_l
     the event frames + LDATI of batch i, results leave on a copy stream).  Returns ClipResult with the concatenated
     event stream (timestamps offset per frame, v2ce.py:365) and the uint8 BGR preview frames (clip-global percentile,
     as the reference computes it)."""
-    from .runner import BatchRunner
     assert image_paths is not None or vidcap is not None
     # pano_fn(model, image_units, width): replaces the serial tile loop of a pano batch (dist.py shares the tiles of a
     # window among ranks when a clip has fewer batches than ranks)
@@ -343,60 +419,39 @@ def stream_clip(model, image_paths=None, vidcap=None, infer_type='center', seq_l
     # the identity and the rest of it runs inside the head conv); float image units otherwise
     # (a clip of <= seq_len frames has a negative first start, v2ce.py:150-154: probe a frame that exists)
     probe = np.asarray(_read_window(image_paths, vidcap, max(int(starts[0]), 0), 0))
-    native = (infer_type == 'center' and hasattr(model, 'forward_frames') and probe.dtype == np.uint8 and
-              probe.shape[-2] == height and int(probe.shape[-1] / probe.shape[-2] * height) == probe.shape[-1] and
-              probe.shape[-1] >= width and width % 2 == 0)
-    # frames at another resolution: the raw uint8 frames are uploaded and /255, the cv2-exact bilinear resize, pair
-    # stacking and Normalize run in one kernel (preprocess.image_units_device, bit-identical to the host path) --
-    # SURVEY.md N1.  device_resize=False (or V2CE_DEVICE_RESIZE=0) keeps cv2.resize on the host, float units over PCIe.
+    # device_resize=False (or V2CE_DEVICE_RESIZE=0) keeps cv2.resize on the host, float units over PCIe
     if device_resize is None:
         device_resize = os.environ.get('V2CE_DEVICE_RESIZE', '1') not in ('', '0')
-    raw = (not native and device_resize and probe.dtype == np.uint8 and probe.ndim == 3 and probe.shape[-2] >= 2)
-    if native:
-        infer = None
+    route, infer = _frame_route(model, infer_type, probe.dtype, probe.shape, height, width, device_resize, pano)
+    if route == 'native':
         batches = _window_batches_u8(image_paths, vidcap, seq_len, batch_size, schedule, width)
-    elif raw:
-        from .preprocess import image_units_device
-        tile = _center_device if infer_type == 'center' else pano
-        infer = lambda u8: tile(model, image_units_device(u8, height), width)        # noqa: E731
+    elif route == 'raw':
         batches = _window_batches_u8(image_paths, vidcap, seq_len, batch_size, schedule, None)
     else:
         infer = (lambda u: _center_device(model, u, width)) if infer_type == 'center' else \
                 (lambda u: pano(model, u, width))
         batches = _batches(image_paths, vidcap, seq_len, height, batch_size, schedule)
-    with torch.cuda.device(device):
-        # the runner owns ~0.5 GB of pinned staging buffers whose allocation costs more than a short clip's compute:
-        # one per (model, device), reused across calls
-        cache = model.__dict__.setdefault('_v2ce_runners', {})
-        runner = cache.get(str(device))
-        if runner is None:
-            runner = cache[str(device)] = BatchRunner(model, device, per_batch_frames=False, copy_out=False,
-                                                      collect_on_device=True)
-        runner.fps, runner.ceil, runner.percentile, runner.keep, runner.seed = fps, ceil, upper_bound_percentile, keep_polarity, seed
-        runner.infer = infer
-        runner.sums = []
-        runner.reset_collection()
-        runner.clip_pairs = int(len(starts) * seq_len - ((seq_len - mode) if mode else 0))
-        pair_idx = pair_base
-        prev = None
-        for x, is_last in _background(batches):
-            t = runner.submit(x if x.is_pinned() else x.pin_memory(), pair_idx, keep_sums=write_event_frames or keep_event_frame_sums,
-                              trim_last_window_to=mode if (is_last and mode != 0) else 0)
-            pair_idx += t.n_pairs
+    plan = batch_plan(starts, mode, batch_size)
+    _claim_model(model)
+    try:
+        with torch.cuda.device(device):
+            clip = _ClipRun(model, device, infer, fps, ceil, upper_bound_percentile, keep_polarity, seed, pair_base,
+                           keep_sums=write_event_frames or keep_event_frame_sums, hand_out=False,
+                           clip_pairs=int(len(starts) * seq_len - ((seq_len - mode) if mode else 0)))
+            runner = clip.runner
+            prev = None
+            for (x, _last), (_a, _e, trim) in zip(_background(batches), plan):
+                t = clip.submit(x if x.is_pinned() else x.pin_memory(), trim)
+                if prev is not None:
+                    runner.wait(prev)                 # status check; the events stay on the device until the end
+                prev = t
             if prev is not None:
-                runner.wait(prev)                 # status check; the events stay on the device until the end
-            prev = t
-        if prev is not None:
-            runner.wait(prev)
-        events_dev, stream = runner.collected_events(to_host=events_to_host)   # False: ClipResult.event_stream is None
-        frames, ub, sums = None, None, None
-        if write_event_frames or keep_event_frame_sums:
-            torch.cuda.current_stream(device).wait_stream(runner.post_stream)
-            sums = torch.cat(runner.sums, dim=0) if len(runner.sums) > 1 else runner.sums[0]
-        if write_event_frames:
-            ub = _ef.upper_bound(sums, upper_bound_percentile, ceil, keep_polarity)
-            frames = _ef.normalize(sums, ub, keep_polarity).cpu().numpy()
-    res = ClipResult(stream, frames, ub, pair_idx - pair_base)
+                runner.wait(prev)
+            events_dev, stream = runner.collected_events(to_host=events_to_host)   # False: ClipResult.event_stream is None
+            frames, ub, sums = clip.event_frames(write_event_frames)
+    finally:
+        _release_model(model)
+    res = ClipResult(stream, frames, ub, clip.pair_idx - pair_base)
     res.ef_sums_dev = sums if keep_event_frame_sums else None   # a sharded clip takes its percentile over all ranks (dist.py)
     res.event_stream_dev = events_dev            # the same bytes on the device (dist.py gathers from here)
     res.n_events = 0 if events_dev is None else events_dev.numel() // 13
